@@ -262,8 +262,10 @@ def close_engines(models):
         UNetEngine.invalidate(m)
 
 
-def device_resident(teacher, students, cfg, scales, S, K, W, dev, precision, rank, world, barrier, max_over_ranks, clock=None):
-    """W untimed + K timed run_chunk calls on pre-staged chunks; returns (ms total, max over ranks)."""
+def device_resident(teacher, students, cfg, scales, S, K, W, dev, precision, rank, world, barrier, max_over_ranks, clock=None,
+                    last=None):
+    """W untimed + K timed run_chunk calls on pre-staged chunks; returns (ms total, max over ranks).  ``last`` (dict): receives
+    what the last timed call returned (red, w1) and its trajectories (the out_traj views, valid until the samplers run again)."""
     import torch
     from distillation_trajectories_b200 import grid
     chunks = [grid.stage_chunk([(i * world + rank) * S + j for j in range(S)], cfg, scales, dev) for i in range(W + K)]
@@ -275,10 +277,36 @@ def device_resident(teacher, students, cfg, scales, S, K, W, dev, precision, ran
     with (clock if clock is not None else contextlib.nullcontext()):
         e0.record()
         for i in range(K):
-            grid.run_chunk(teacher, students, chunks[W + i], dev, precision)
+            traj = []
+            red, w1, _ = grid.run_chunk(teacher, students, chunks[W + i], dev, precision, out_traj=traj)
         e1.record()
         barrier()
+    if last is not None:
+        last.update(red=red, w1=w1, traj=traj)
     return max_over_ranks(e0.elapsed_time(e1))
+
+
+DUMP_ROWS = 512         # 512 (seed, guidance) pairs of 1x16x16 frames: 54 MB of .npy files
+
+
+def dump_outputs(out_dir, red, w1, traj):
+    """--dump-outputs: what the last timed step returned, as float32 .npy files: the pair reductions red.npy [n_students, n, L, 6],
+    the per-frame Wasserstein distances w1.npy [n_students, n, L] and the frames behind them, teacher_traj.npy and
+    student<i>_traj.npy [n, L, D].  n = the same fixed sample (RandomState(0)) of at most DUMP_ROWS of the step's N pairs in every
+    array, in ascending pair order; the whole step's trajectories are too large to keep."""
+    import numpy as np
+    import torch
+    n_pairs = red.shape[1]
+    rows = np.sort(np.random.RandomState(0).choice(n_pairs, min(n_pairs, DUMP_ROWS), replace=False))
+    idx = torch.from_numpy(rows).to(red.device)
+    arrays = {"red": red[:, idx], "w1": w1[:, idx], "teacher_traj": traj[0][0][idx]}
+    arrays.update({f"student{i}_traj": s[idx] for i, (_, s) in enumerate(traj)})
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs would write {total / 2**20:.0f} MiB"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def conv_flops_per_forward(dims, C, H, executed, skip_enc1=False):
@@ -463,7 +491,11 @@ def run_ours(args, emit=print):
 
     # ---- headline: device-resident leg, then the end-to-end leg (public sweep API, host-side inputs)
     clk = ClockSampler(local)
-    ms = device_resident(teacher, [student], Cfg, GUIDANCE, S, K, W, dev, args.precision, rank, world, barrier, max_over_ranks, clk)
+    last = {}
+    ms = device_resident(teacher, [student], Cfg, GUIDANCE, S, K, W, dev, args.precision, rank, world, barrier, max_over_ranks, clk,
+                         last)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, **last)
     value = traj_per_step * K / (ms / 1e3)
     samplers = samplers_of(models, Cfg, args.precision, dev)
     launches = K * (sum(s.launches for s in samplers) + 2)
@@ -712,7 +744,12 @@ def main():
     ap.add_argument("--ref-seeds", type=int, default=1, help="--impl reference: seeds per step (x 8 scales x 2 models)")
     ap.add_argument("--config3-seeds", type=int, default=1024, help="seeds per chunk of the configs[2] leg (0 = skip)")
     ap.add_argument("--config4-seeds", type=int, default=9472, help="TOTAL seeds of the configs[3]-shaped strong-scaling slice (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs: it cannot be combined with --impl reference")
     if args.quick:
         args.config4_seeds = 0
     if args.impl == "reference":

@@ -288,25 +288,28 @@ def test_staged_reference_is_byte_identical_and_complete():
 
 
 def test_model_aliases_match_the_reference_constructors():
-    """M4 (models.py:227-242): SimpleUNet / StudentUNet create the same parameters as the reference's aliases."""
-    from oracle import refload
-    if not refload.available():
-        pytest.skip("reference tree not present")
+    """M4 (models.py:227-242): SimpleUNet / StudentUNet create the same parameters as the reference's aliases: the names, shapes,
+    per-tensor sums and widths stored in tests/golden/reference_checks.npz, and the reference's own parameters when present."""
     import contextlib
     import io
-    from distillation_trajectories_b200 import models as ours
-    ref = refload.load()
+    from oracle import make_golden_reference_checks as mk
+    from oracle import refload
+    g = load_golden("reference_checks")
     cfg = refload.RefConfig(1, 16, 8)
-    for mk_ref, mk_ours in ((lambda: ref.models.SimpleUNet(cfg), lambda: ours.SimpleUNet(cfg)),
-                            (lambda: ref.models.StudentUNet(cfg, 0.3, "tiny"), lambda: ours.StudentUNet(cfg, 0.3, "tiny"))):
+    ref = refload.load() if refload.available() else None
+    for which in ("simple", "student"):
         with contextlib.redirect_stdout(io.StringIO()):
             torch.manual_seed(4)
-            a = mk_ref()
-            torch.manual_seed(4)
-            b = mk_ours()
-        sa, sb = a.state_dict(), b.state_dict()
-        assert list(sa) == list(sb) and all(torch.equal(sa[k], sb[k]) for k in sa)
-        assert a.dims == b.dims and a.time_emb_dim == b.time_emb_dim
+            b = mk.ours_alias(cfg, which)
+            if ref is not None:
+                torch.manual_seed(4)
+                a = ref.models.SimpleUNet(cfg) if which == "simple" else ref.models.StudentUNet(cfg, 0.3, "tiny")
+        if ref is not None:             # the reference's own constructors, in this process: exact
+            sa, sb = a.state_dict(), b.state_dict()
+            assert list(sa) == list(sb) and all(torch.equal(sa[k], sb[k]) for k in sa)
+            assert a.dims == b.dims and a.time_emb_dim == b.time_emb_dim
+        mk.check_weights(b, g, f"alias/{which}/weights/")
+        assert list(b.dims) == list(g[f"alias/{which}/dims"]) and b.time_emb_dim == int(g[f"alias/{which}/time_emb_dim"]), which
 
 
 def test_bench_flop_counts_match_the_survey_and_the_reference_layers():
