@@ -355,11 +355,11 @@ extern "C" int dtraj_unet_time_bias(const dtraj_unet* u, int32_t t, int32_t vari
 // Optional per-launch timing (dtraj_sampler_profile): one event pair per launch, summed per class.
 enum KernelClass : int { KC_CONV = 0, KC_FIRST = 1, KC_RESAMPLE = 2, KC_STEP = 3, KC_ENC1 = 4, KC_COUNT = 5 };
 struct Profiler {
-    struct Rec { int cls; cudaEvent_t a, b; const char* name; int step; unsigned grid; double flops; };
+    struct Rec { int cls; cudaEvent_t a, b; const char* name; int step; unsigned grid; double flops; float ms; };
     std::vector<Rec> recs;
     cudaStream_t st = nullptr;
     int step = 0;               // sampler step the launches belong to
-    void begin(int cls, const char* name = "", unsigned grid = 0, double flops = 0.0) {
+    void begin(int cls, const char* name, unsigned grid, double flops) {
         Rec r; r.cls = cls; r.name = name; r.step = step; r.grid = grid; r.flops = flops;
         cudaEventCreate(&r.a); cudaEventCreate(&r.b);
         cudaEventRecord(r.a, st);
@@ -367,8 +367,26 @@ struct Profiler {
     }
     void end() { cudaEventRecord(recs.back().b, st); }
 };
-#define PROF_BEGIN(prof, ...) do { if (prof) (prof)->begin(__VA_ARGS__); } while (0)
-#define PROF_END(prof) do { if (prof) (prof)->end(); } while (0)
+
+// One kernel launch of a forward.  plan_build decides the kernel and builds its parameters once; plan_forward writes only
+// the per-call inputs (frame, row tables, time-table row) into the fields the kind reads, and launches.
+struct Launch {
+    enum Kind : int { ENC1H, ENC1, FIRST, CONV_UMMA, CONV_SIMT, POOL, POOL_H, UP, UP_H, UP_H4, FINAL };
+    Kind kind;
+    KernelClass cls;
+    char name[40];              // profiler name
+    unsigned grid;              // CTAs (0 for CONV_SIMT: launch_conv_simt chooses its 2-d grid)
+    double flops;               // executed tensor-core flops, real channels (KC_CONV, KC_ENC1)
+    int tb_block = -1;          // block whose time-bias row this launch reads, -1: none
+    Enc1hLaunch enc1h;          // ENC1H
+    Enc1Launch enc1;            // ENC1
+    FirstConvParams first; size_t first_smem;   // FIRST and its dynamic shared memory
+    UmmaLaunch U;               // CONV_UMMA
+    ConvLayer L;                // CONV_SIMT
+    struct {                    // POOL*, UP*, FINAL: n = the kernel's element count, cv = channel vectors per pixel
+        const float* in; float* out; int64_t n; int S, cv, lg_s, lg_cv; int64_t lo_off; int act_mode; Up2Coef cf;
+    } rs;
+};
 
 struct dtraj_plan {
     const dtraj_unet* u = nullptr;
@@ -377,20 +395,7 @@ struct dtraj_plan {
     // buffers (float offsets into ws); lo planes follow at +size when act_mode == ACT_SPLIT
     struct Buf { float* p = nullptr; int64_t n = 0; int64_t lo = 0; };
     Buf tmp_h, tmp_r, tmp_x, p1, x2, p2, x3, p3, x4, p4, u3, u2, u1, y1, elow;
-    // generic conv launches in execution order
-    struct ConvOp { ConvLayer L; bool umma; UmmaLaunch U; int tb_block; double flops; bool needs_x; char name[40]; };
-    // fused tails (single-pass TF32 mode): which stand-alone kernels the conv epilogues replace
-    bool fuse_resx = false, fuse_final = false;
-    bool fuse_res[8] = {false, false, false, false, false, false, false, false};   // per block: its 1x1 residual conv rides in conv2's launch
-    // execution order of one forward after the enc1 stage: generic convs, stand-alone pools, upsamples
-    struct Op { int kind; int a; };     // kind 0: next conv; 1: pool after encoder level a; 2: upsample of decoder stage a (0..2)
-    std::vector<Op> seq;
-    bool fuse_enc1 = false;      // k_enc1_umma replaces k_conv_first + the enc1.conv2 launch
-    Enc1Launch enc1;
-    Enc1hLaunch enc1h;           // its fp16 form (DTRAJ_PREC_F16): conv2 weights resident in shared memory
-    bool fuse_pool[4] = {false, false, false, false};   // pool after enc1..enc4
-    std::vector<ConvOp> convs;   // 15 3x3 + residual 1x1s
-    int64_t launches_per_forward = 0;
+    std::vector<Launch> launches;   // one forward, in execution order
 };
 
 namespace {
@@ -444,12 +449,23 @@ struct Tail {                // optional fused epilogue tails of one conv
     const dtraj_plan::Buf* rs1 = nullptr;
 };
 
+inline unsigned blocks_for(int64_t n, int per) { return (unsigned)((n + per - 1) / per); }
+
+// appends a zeroed launch record to the plan; the caller fills in the kind's parameters
+Launch& add_launch(dtraj_plan* P, Launch::Kind kind, KernelClass cls, const char* name, unsigned grid = 0) {
+    P->launches.emplace_back();
+    Launch& l = P->launches.back();
+    l.kind = kind; l.cls = cls; l.grid = grid;
+    snprintf(l.name, sizeof(l.name), "%s", name);
+    return l;
+}
+
 int add_conv(dtraj_plan* P, const char* name, const PackedConv& pc, const dtraj_plan::Buf& s0, const dtraj_plan::Buf* s1, int S,
              const dtraj_plan::Buf& out, const float* resid, int flags, int tb_block, bool is_residual_conv,
              const Tail& tail = Tail()) {
     const dtraj_unet* u = P->u;
-    dtraj_plan::ConvOp op;
-    memset(&op.L, 0, sizeof(op.L));
+    const bool umma = u->d.precision != DTRAJ_PREC_FP32;
+    Launch& op = add_launch(P, umma ? Launch::CONV_UMMA : Launch::CONV_SIMT, KC_CONV, "");
     ConvLayer& L = op.L;
     L.src0 = s0.p; L.src0_lo = s0.p + s0.lo; L.c0p = pc.c0p;
     if (s1) { L.src1 = s1->p; L.src1_lo = s1->p + s1->lo; L.c1p = pc.c1p; }
@@ -463,13 +479,11 @@ int add_conv(dtraj_plan* P, const char* name, const PackedConv& pc, const dtraj_
     L.f16 = u->d.precision == DTRAJ_PREC_F16 ? 1 : 0;
     L.err = u->err;
     snprintf(op.name, sizeof(op.name), "%s%s%s%s", name, tail.res ? " +res" : "", tail.pool_out ? " +pool" : "", tail.final1x1 ? " +final" : "");
-    op.needs_x = false;
     if (tail.pool_out) { L.flags |= CONV_POOL; L.pool_out = tail.pool_out; }
     if (tail.nostore) L.flags |= CONV_NOSTORE;
     if (tail.resx) {
         L.flags |= CONV_RESX;
         L.rw1 = u->fw1; L.rb1 = u->fb1; L.xC = u->d.channels;
-        op.needs_x = true;
     }
     if (tail.final1x1) {
         L.flags |= CONV_FINAL;
@@ -484,15 +498,15 @@ int add_conv(dtraj_plan* P, const char* name, const PackedConv& pc, const dtraj_
         L.rbias = tail.res->bias;
         op.flops += 2.0 * (double)L.M * tail.res->cout * (double)(tail.res->c0 + tail.res->c1);
     }
-    op.umma = u->d.precision != DTRAJ_PREC_FP32;
-    if (op.umma) DTRAJ_TRY(build_umma_launch(&op.U, L, u->d.precision == DTRAJ_PREC_TF32X3 ? 3 : 1, pc.w, pc.rows,
-                                             tail.res ? tail.res->w : nullptr, tail.res ? tail.res->rows : 0));
-    if (op.umma && op.U.conv.posm) {    // position-major tiles skip the taps outside the map: ((3H - 2) / H)^2 of 9 are executed on average
+    if (!umma) return 0;
+    DTRAJ_TRY(build_umma_launch(&op.U, L, u->d.precision == DTRAJ_PREC_TF32X3 ? 3 : 1, pc.w, pc.rows,
+                                tail.res ? tail.res->w : nullptr, tail.res ? tail.res->rows : 0));
+    op.grid = op.U.grid;
+    if (op.U.conv.posm) {    // position-major tiles skip the taps outside the map: ((3H - 2) / H)^2 of 9 are executed on average
         const double t_eff = ((3.0 * L.H - 2.0) / L.H) * ((3.0 * L.W - 2.0) / L.W);
         op.flops = 2.0 * (double)L.M * pc.cout * (double)(pc.c0 + pc.c1) * t_eff +
                    (tail.res ? 2.0 * (double)L.M * tail.res->cout * (double)(tail.res->c0 + tail.res->c1) : 0.0);
     }
-    P->convs.push_back(op);
     return 0;
 }
 
@@ -505,65 +519,116 @@ int plan_build(const dtraj_unet* u, int64_t R, void* ws, int64_t ws_bytes, dtraj
     P->u = u; P->R = R; P->ws = (float*)ws;
     plan_floats(u, R, P);
     const int* S = u->sizes;
+    const int* dp = u->dp;
+    const int C = u->d.channels;
     int rc = 0;
     const int RT = CONV_RELU | CONV_TBIAS, RR = CONV_RELU | CONV_RESID;
     auto blk = [&](int b) -> const BlockW& { return u->blk[b]; };
+    auto conv = [&](auto&&... a) { if (!rc) rc = add_conv(P, a...); };
     // Fused epilogue tails exist in the tcgen05 kernel's bulk path only (single-pass TF32, the mode the
     // sweeps run in); the exact modes keep the stand-alone pool / final / residual kernels.
     const bool f16 = u->d.precision == DTRAJ_PREC_F16;
     const bool fused = f16 || u->d.precision == DTRAJ_PREC_TF32;
-    P->fuse_resx = fused;
-    P->fuse_final = fused;
+    const bool fuse_resx = fused, fuse_final = fused;
     // (maps of at most 4x4 run position-major tiles -- csrc/conv_umma.cuh -- whose rows are images, so a 2x2 pool window is not
     //  inside one tile: those levels keep the stand-alone pool kernel)
-    for (int l = 0; l < 4; ++l) P->fuse_pool[l] = fused && S[l] <= 16 && !umma_posm_applies(S[l], P->R);
+    bool fuse_pool[4];           // pool after enc1..enc4
+    for (int l = 0; l < 4; ++l) fuse_pool[l] = fused && S[l] <= 16 && !umma_posm_applies(S[l], R);
     // Residual 1x1 convs as extra MMAs of the block's conv2 (CONV_RESACC): no r tensor, no extra launch.  (Measured in round 2
     // with the 1x1 convs of the 256-wide blocks as their own launches + the TMA residual path: conv2 alone gains -- enc2.conv2
     // 673 -> 454 us at 8880 rows, two accumulator stages instead of one -- but the stand-alone K = 128..512 GEMMs cost more than
     // that, 3579 vs 3499 us per teacher forward; profiles/r02b_resacc_ab.txt.)
-    for (int b = 1; b < 8; ++b) P->fuse_res[b] = fused && blk(b).has_res;
+    bool fuse_res[8] = {};
+    for (int b = 1; b < 8; ++b) fuse_res[b] = fused && blk(b).has_res;
     auto with_res = [&](Tail t, int b, const dtraj_plan::Buf* s0, const dtraj_plan::Buf* s1) {
-        if (P->fuse_res[b]) { t.res = &u->blk[b].res; t.rs0 = s0; t.rs1 = s1; }
+        if (fuse_res[b]) { t.res = &u->blk[b].res; t.rs0 = s0; t.rs1 = s1; }
         return t;
     };
     const dtraj_plan::Buf* pooled[4] = {&P->p1, &P->p2, &P->p3, &P->p4};
     auto tail_for = [&](int enc) {   // conv2 of encoder block `enc` (0..3)
         Tail t;
-        if (P->fuse_pool[enc]) t.pool_out = pooled[enc]->p;
+        if (fuse_pool[enc]) t.pool_out = pooled[enc]->p;
         return t;
     };
-#define ADD(...) do { if (!rc) { rc = add_conv(P, __VA_ARGS__); P->seq.push_back({0, 0}); } } while (0)
+    // a stand-alone pool / upsample over n4 4-channel vectors (the fp16 kernels take 8-channel ones)
+    auto resample = [&](Launch::Kind kind_h, Launch::Kind kind, const char* name, const dtraj_plan::Buf& in,
+                        const dtraj_plan::Buf& o, int64_t n4, int S_in, int cp, int act_mode) {
+        Launch& r = add_launch(P, f16 ? kind_h : kind, KC_RESAMPLE, name, blocks_for(f16 ? n4 / 2 : n4, 256));
+        r.rs.in = in.p; r.rs.out = o.p; r.rs.n = f16 ? n4 / 2 : n4; r.rs.S = S_in; r.rs.cv = cp / (f16 ? 8 : 4);
+        r.rs.lo_off = o.lo; r.rs.act_mode = act_mode;
+    };
+    // 2x2 max-pool after encoder level `lv`, unless the producing conv's epilogue emits it
+    const dtraj_plan::Buf* pool_in[4] = {&P->tmp_x, &P->x2, &P->x3, &P->x4};
+    auto pool = [&](int lv) {
+        const int So = S[lv + 1];
+        if (!fuse_pool[lv])
+            resample(Launch::POOL_H, Launch::POOL, "maxpool 2x2", *pool_in[lv], *pooled[lv], R * So * So * (dp[lv] / 4), So, dp[lv],
+                     pooled[lv]->lo ? ACT_SPLIT : ACT_PLAIN);
+    };
+    // bilinear x2 upsample of the map below decoder stage k (0..2) into its first input
+    const dtraj_plan::Buf* up[3] = {&P->u3, &P->u2, &P->u1};
+    auto upsample = [&](int k) -> int {
+        const int Si = S[4 - k], cp = dp[3 - k], cp8 = cp / 8;
+        const int64_t n4 = R * (2 * Si) * (2 * Si) * (cp / 4);
+        if (n4 >= ((int64_t)1 << 31)) return fail(DTRAJ_EINVAL, "upsample: batch too large for 32-bit indexing");
+        const std::string name = "upsample " + std::to_string(Si) + "->" + std::to_string(2 * Si);
+        Up2Coef cf;
+        if (!(f16 && (cp8 & (cp8 - 1)) == 0 && up2_static_ok(Si, &cf))) {
+            resample(Launch::UP_H, Launch::UP, name.c_str(), P->tmp_x, *up[k], n4, Si, cp,
+                     (u->act_mode == ACT_SPLIT && !up[k]->lo) ? ACT_PLAIN : u->act_mode);
+            return 0;
+        }
+        const int64_t n_blk = R * Si * Si * cp8;
+        Launch& r = add_launch(P, Launch::UP_H4, KC_RESAMPLE, name.c_str(), blocks_for(n_blk, 256));
+        r.rs.in = P->tmp_x.p; r.rs.out = up[k]->p; r.rs.n = n_blk; r.rs.S = Si; r.rs.cv = cp8; r.rs.cf = cf;
+        while ((1 << r.rs.lg_s) < Si) ++r.rs.lg_s;
+        while ((1 << r.rs.lg_cv) < cp8) ++r.rs.lg_cv;
+        return 0;
+    };
     // enc1: conv1/res by k_conv_first; conv2 here.  x1 itself is never a skip input (models.py:206-216):
     // with the pool fused, only the pooled tile is written.
-    P->fuse_enc1 = fused && S[0] % 16 == 0 && u->d.channels <= 4;
-    if (f16 && u->dp[0] > 128) P->fuse_enc1 = false;   // the fp16 fused kernel holds D1 + two accumulators in TMEM: widths up to 128;
-                                                        // wider first blocks take k_conv_first + the generic conv2 (RESX + POOL tails)
-    if (P->fuse_enc1 && f16) {
-        rc = build_enc1h_launch(&P->enc1h, u->d.channels, S[0], u->dp[0], blk(0).cout, P->R, blk(0).conv2.w, blk(0).conv2.rows);
-        Enc1hParams& e = P->enc1h.p;
+    bool fuse_enc1 = fused && S[0] % 16 == 0 && C <= 4;   // k_enc1_umma / k_enc1_f16 replace k_conv_first + the enc1.conv2 launch
+    if (f16 && dp[0] > 128) fuse_enc1 = false;   // the fp16 fused kernel holds D1 + two accumulators in TMEM: widths up to 128;
+                                                 // wider first blocks take k_conv_first + the generic conv2 (RESX + POOL tails)
+    auto enc1_fused = [&](Launch& l, auto& E) {   // what the two fused enc1 launches (Enc1hLaunch, Enc1Launch) share
+        auto& e = E.p;
         e.w3 = u->fw3; e.b3 = u->fb3; e.rw1 = u->fw1; e.rb1 = u->fb1; e.bias2 = blk(0).conv2.bias;
-        e.tb_var_stride = u->tb_stride; e.pool_out = (__half*)P->p1.p; e.err = u->err;
-    } else if (P->fuse_enc1) {
-        rc = build_enc1_launch(&P->enc1, u->d.channels, S[0], u->dp[0], blk(0).cout, P->R, blk(0).conv2.w, blk(0).conv2.rows);
-        Enc1Params& e = P->enc1.p;
-        e.w3 = u->fw3; e.b3 = u->fb3; e.rw1 = u->fw1; e.rb1 = u->fb1; e.bias2 = blk(0).conv2.bias;
-        e.tb_var_stride = u->tb_stride; e.pool_out = P->p1.p; e.act_mode = u->act_mode; e.err = u->err;
-    } else {
+        e.tb_var_stride = u->tb_stride; e.pool_out = (decltype(e.pool_out))P->p1.p; e.err = u->err;
+        l.grid = E.grid; l.flops = E.flops; l.tb_block = 0;
+    };
+    if (fuse_enc1 && f16) {      // conv2 weights resident in shared memory
+        Launch& l = add_launch(P, Launch::ENC1H, KC_ENC1, "enc1 fused (k_enc1_f16)");
+        rc = build_enc1h_launch(&l.enc1h, C, S[0], dp[0], blk(0).cout, R, blk(0).conv2.w, blk(0).conv2.rows);
+        enc1_fused(l, l.enc1h);
+    } else if (fuse_enc1) {      // whole enc1 block + pool in one kernel
+        Launch& l = add_launch(P, Launch::ENC1, KC_ENC1, "enc1 fused (k_enc1_umma)");
+        rc = build_enc1_launch(&l.enc1, C, S[0], dp[0], blk(0).cout, R, blk(0).conv2.w, blk(0).conv2.rows);
+        enc1_fused(l, l.enc1);
+        l.enc1.p.act_mode = u->act_mode;
+    } else {                     // enc1.conv1 + residual
+        Launch& l = add_launch(P, Launch::FIRST, KC_FIRST, "enc1.conv1 + res (k_conv_first)", (unsigned)R);
+        FirstConvParams& f = l.first;
+        f.C = C; f.H = S[0]; f.W = S[0]; f.coutp = dp[0];
+        f.w3 = u->fw3; f.b3 = u->fb3; f.w1 = u->fw1; f.b1 = u->fb1; f.tb_var_stride = u->tb_stride;
+        f.h = P->tmp_h.p; f.r = fuse_resx ? nullptr : P->tmp_r.p; f.lo_off = P->tmp_h.lo;
+        f.f16 = f16 ? 1 : 0; f.act_mode = f16 ? ACT_PLAIN : u->act_mode;
+        l.first_smem = (round_up(C * (S[0] + 2) * (S[0] + 2), 4) + 10 * C * dp[0]) * sizeof(float);
+        l.tb_block = 0;
         Tail t = tail_for(0);
-        t.resx = P->fuse_resx;
-        t.nostore = P->fuse_pool[0];
-        ADD("enc1.conv2", blk(0).conv2, P->tmp_h, nullptr, S[0], P->tmp_x, t.resx ? nullptr : P->tmp_r.p, t.resx ? CONV_RELU : RR, -1, false, t);
+        t.resx = fuse_resx;
+        t.nostore = fuse_pool[0];
+        conv("enc1.conv2", blk(0).conv2, P->tmp_h, nullptr, S[0], P->tmp_x, t.resx ? nullptr : P->tmp_r.p, t.resx ? CONV_RELU : RR, -1, false, t);
+        pool(0);
     }
-    if (!P->fuse_enc1) P->seq.push_back({1, 0});
     // enc2 @ level 1
     if (!blk(1).has_res) rc = fail(DTRAJ_EINVAL, "enc2 without residual_conv unsupported");
     {
-        const bool fr = P->fuse_res[1];
-        if (!fr) ADD("enc2.res", blk(1).res, P->p1, nullptr, S[1], P->tmp_r, nullptr, 0, -1, true);
-        ADD("enc2.conv1", blk(1).conv1, P->p1, nullptr, S[1], P->tmp_h, nullptr, RT, 1, false);
-        ADD("enc2.conv2", blk(1).conv2, P->tmp_h, nullptr, S[1], P->x2, fr ? nullptr : P->tmp_r.p, fr ? CONV_RELU : RR, -1, false,
-            with_res(tail_for(1), 1, &P->p1, nullptr));
-        P->seq.push_back({1, 1});
+        const bool fr = fuse_res[1];
+        if (!fr) conv("enc2.res", blk(1).res, P->p1, nullptr, S[1], P->tmp_r, nullptr, 0, -1, true);
+        conv("enc2.conv1", blk(1).conv1, P->p1, nullptr, S[1], P->tmp_h, nullptr, RT, 1, false);
+        conv("enc2.conv2", blk(1).conv2, P->tmp_h, nullptr, S[1], P->x2, fr ? nullptr : P->tmp_r.p, fr ? CONV_RELU : RR, -1, false,
+             with_res(tail_for(1), 1, &P->p1, nullptr));
+        pool(1);
     }
     // enc3, enc4, bottleneck @ levels 2..4 (identity residual = the pooled input, unless the widths differ)
     const dtraj_plan::Buf* pin[3] = {&P->p2, &P->p3, &P->p4};
@@ -571,151 +636,104 @@ int plan_build(const dtraj_unet* u, int64_t R, void* ws, int64_t ws_bytes, dtraj
     for (int k = 0; k < 3 && !rc; ++k) {
         const int b = 2 + k, lv = 2 + k;
         const float* resid = pin[k]->p;
-        const bool fused_here = P->fuse_res[b];
+        const bool fused_here = fuse_res[b];
         const std::string bn = kBlockNames[b];
-        if (blk(b).has_res && !fused_here) { ADD((bn + ".res").c_str(), blk(b).res, *pin[k], nullptr, S[lv], P->tmp_r, nullptr, 0, -1, true); resid = P->tmp_r.p; }
-        ADD((bn + ".conv1").c_str(), blk(b).conv1, *pin[k], nullptr, S[lv], P->tmp_h, nullptr, RT, b, false);
-        ADD((bn + ".conv2").c_str(), blk(b).conv2, P->tmp_h, nullptr, S[lv], *xo[k], fused_here ? nullptr : resid, fused_here ? CONV_RELU : RR, -1, false,
-            with_res(k < 2 ? tail_for(2 + k) : Tail(), b, pin[k], nullptr));
-        if (k < 2) P->seq.push_back({1, 2 + k});
+        if (blk(b).has_res && !fused_here) { conv((bn + ".res").c_str(), blk(b).res, *pin[k], nullptr, S[lv], P->tmp_r, nullptr, 0, -1, true); resid = P->tmp_r.p; }
+        conv((bn + ".conv1").c_str(), blk(b).conv1, *pin[k], nullptr, S[lv], P->tmp_h, nullptr, RT, b, false);
+        conv((bn + ".conv2").c_str(), blk(b).conv2, P->tmp_h, nullptr, S[lv], *xo[k], fused_here ? nullptr : resid, fused_here ? CONV_RELU : RR, -1, false,
+             with_res(k < 2 ? tail_for(2 + k) : Tail(), b, pin[k], nullptr));
+        if (k < 2) pool(2 + k);
     }
     // decoders: [upsampled | skip]
-    const dtraj_plan::Buf* up[3] = {&P->u3, &P->u2, &P->u1};
     const dtraj_plan::Buf* skip[3] = {&P->x4, &P->x3, &P->x2};
     const dtraj_plan::Buf* yo[3] = {&P->tmp_x, &P->tmp_x, &P->y1};
     for (int k = 0; k < 3 && !rc; ++k) {
         const int b = 5 + k, lv = 3 - k;
         if (!blk(b).has_res) { rc = fail(DTRAJ_EINVAL, "%s without residual_conv unsupported", kBlockNames[b]); break; }
         const std::string bn = kBlockNames[b];
-        const bool fr = P->fuse_res[b];
-        P->seq.push_back({2, k});
-        if (!fr) ADD((bn + ".res").c_str(), blk(b).res, *up[k], skip[k], S[lv], P->tmp_r, nullptr, 0, -1, true);
-        ADD((bn + ".conv1").c_str(), blk(b).conv1, *up[k], skip[k], S[lv], P->tmp_h, nullptr, RT, b, false);
+        const bool fr = fuse_res[b];
+        rc = upsample(k);
+        if (!fr) conv((bn + ".res").c_str(), blk(b).res, *up[k], skip[k], S[lv], P->tmp_r, nullptr, 0, -1, true);
+        conv((bn + ".conv1").c_str(), blk(b).conv1, *up[k], skip[k], S[lv], P->tmp_h, nullptr, RT, b, false);
         Tail t;
-        if (k == 2 && P->fuse_final) { t.final1x1 = true; t.nostore = true; }   // y1 only feeds the final 1x1
-        ADD((bn + ".conv2").c_str(), blk(b).conv2, P->tmp_h, nullptr, S[lv], *yo[k], fr ? nullptr : P->tmp_r.p, fr ? CONV_RELU : RR, -1, false,
-            with_res(t, b, up[k], skip[k]));
+        if (k == 2 && fuse_final) { t.final1x1 = true; t.nostore = true; }   // y1 only feeds the final 1x1
+        conv((bn + ".conv2").c_str(), blk(b).conv2, P->tmp_h, nullptr, S[lv], *yo[k], fr ? nullptr : P->tmp_r.p, fr ? CONV_RELU : RR, -1, false,
+             with_res(t, b, up[k], skip[k]));
     }
-#undef ADD
+    if (!fuse_final) {   // final 1x1 at half resolution (else: dec1.conv2's epilogue)
+        const int64_t npix = R * S[1] * S[1];
+        Launch& r = add_launch(P, Launch::FINAL, KC_RESAMPLE, "final 1x1", blocks_for(npix * 32, 256));
+        r.rs.in = P->y1.p; r.rs.out = P->elow.p; r.rs.n = npix; r.rs.cv = dp[0];
+    }
     if (rc) { delete P; return rc; }
     *out = P;
     return 0;
 }
 
-inline unsigned blocks_for(int64_t n, int per) { return (unsigned)((n + per - 1) / per); }
+// Writes the per-call inputs into the fields launch `l` reads and launches it.  `tbias`: the time-table row of this call's
+// t at the record's block (null when it reads none).
+int launch_record(Launch& l, const dtraj_unet* u, const float* x, int64_t x_stride, const int32_t* row_sample,
+                  const int32_t* row_variant, const float* tbias, bool per_row, cudaStream_t st) {
+    const auto& r = l.rs;
+    auto enc1_inputs = [&](auto& p) {   // Enc1hParams, Enc1Params, FirstConvParams
+        p.x = x; p.x_stride = x_stride; p.row_sample = row_sample; p.row_variant = row_variant; p.tbias = tbias;
+    };
+    switch (l.kind) {
+    case Launch::ENC1H: enc1_inputs(l.enc1h.p); l.enc1h.p.tb_rows = per_row ? 1 : 0; return launch_enc1h(l.enc1h, st);
+    case Launch::ENC1: enc1_inputs(l.enc1.p); return launch_enc1(l.enc1, st);
+    case Launch::FIRST: enc1_inputs(l.first); k_conv_first<<<l.grid, 256, l.first_smem, st>>>(l.first); break;
+    case Launch::CONV_UMMA: {
+        ConvLayer& L = l.U.conv.L;
+        L.tbias = tbias; L.row_variant = row_variant; L.tb_rows = per_row ? 1 : 0;
+        if (L.flags & CONV_RESX) { L.xraw = x; L.x_stride = x_stride; L.row_sample = row_sample; }
+        return launch_conv_umma(l.U, st);
+    }
+    case Launch::CONV_SIMT: l.L.tbias = tbias; l.L.row_variant = row_variant; return launch_conv_simt(l.L, st);
+    case Launch::POOL: k_pool2<<<l.grid, 256, 0, st>>>(r.in, r.out, r.n, r.S, r.S, r.cv, r.lo_off, r.act_mode); break;
+    case Launch::POOL_H: k_pool2_h<<<l.grid, 256, 0, st>>>((const __half*)r.in, (__half*)r.out, r.n, r.S, r.S, r.cv); break;
+    case Launch::UP: k_upsample2<<<l.grid, 256, 0, st>>>(r.in, r.out, r.n, r.S, r.S, r.cv, r.lo_off, r.act_mode); break;
+    case Launch::UP_H:
+        DTRAJ_CUDA(launch_ex(k_upsample2_h, l.grid, 256, 0, st, 1, true, (const __half*)r.in, (__half*)r.out, r.n, r.S, r.S, r.cv));
+        break;
+    case Launch::UP_H4:
+        DTRAJ_CUDA(launch_ex(k_upsample2_h4, l.grid, 256, 0, st, 1, true, (const __half*)r.in, (__half*)r.out, (uint32_t)r.n, r.S,
+                             r.lg_s, r.cv, r.lg_cv, r.cf));
+        break;
+    case Launch::FINAL: k_final1x1<<<l.grid, 256, 0, st>>>(r.in, u->finw, u->finb, r.out, r.n, r.cv, u->d.channels); break;
+    }
+    DTRAJ_LAUNCH_CHECK();
+    return 0;
+}
 
 // Enqueue one U-Net forward (models.py:159-224 up to the half-resolution eps map).
 // `per_row`: row_variant holds t_i * 3 + variant_i (a row of the whole table) instead of the variant alone, `t` is 0.
-int plan_forward(dtraj_plan* P, const float* x, int64_t x_stride, const int32_t* row_sample,
-                 const int32_t* row_variant, int t, cudaStream_t st, int64_t* launches, Profiler* prof = nullptr,
-                 bool per_row = false) {
+int plan_forward(dtraj_plan* P, const float* x, int64_t x_stride, const int32_t* row_sample, const int32_t* row_variant, int t,
+                 bool per_row, cudaStream_t st, Profiler* prof = nullptr) {
     const dtraj_unet* u = P->u;
     if (t < 0 || t >= u->d.n_timesteps) return fail(DTRAJ_EINVAL, "timestep %d outside the time table (0..%d)", t, u->d.n_timesteps - 1);
-    const int* S = u->sizes;
-    const int* dp = u->dp;
-    const int C = u->d.channels;
-    const int64_t R = P->R;
     const float* trow = u->table + (size_t)t * 3 * u->tb_stride;
-    const bool f16 = u->d.precision == DTRAJ_PREC_F16;
-    int64_t nl = 0;
-    if (P->fuse_enc1 && f16) {
-        Enc1hParams& e = P->enc1h.p;
-        e.x = x; e.x_stride = x_stride; e.row_sample = row_sample; e.row_variant = row_variant;
-        e.tbias = trow + u->tb_off[0];
-        e.tb_rows = per_row ? 1 : 0;
-        PROF_BEGIN(prof, KC_ENC1, "enc1 fused (k_enc1_f16)", P->enc1h.grid, P->enc1h.flops);
-        int rc1 = launch_enc1h(P->enc1h, st);
-        PROF_END(prof);
-        DTRAJ_TRY(rc1);
-        ++nl;
-    } else if (P->fuse_enc1) {   // whole enc1 block + pool in one kernel
-        Enc1Params& e = P->enc1.p;
-        e.x = x; e.x_stride = x_stride; e.row_sample = row_sample; e.row_variant = row_variant;
-        e.tbias = trow + u->tb_off[0];
-        PROF_BEGIN(prof, KC_ENC1, "enc1 fused (k_enc1_umma)", P->enc1.grid, P->enc1.flops);
-        int rc1 = launch_enc1(P->enc1, st);
-        PROF_END(prof);
-        DTRAJ_TRY(rc1);
-        ++nl;
-    } else {   // enc1.conv1 + residual
-        FirstConvParams f;
-        f.x = x; f.x_stride = x_stride; f.row_sample = row_sample; f.row_variant = row_variant;
-        f.C = C; f.H = S[0]; f.W = S[0]; f.coutp = dp[0];
-        f.w3 = u->fw3; f.b3 = u->fb3; f.w1 = u->fw1; f.b1 = u->fb1;
-        f.tbias = trow + u->tb_off[0]; f.tb_var_stride = u->tb_stride;
-        f.h = P->tmp_h.p; f.r = P->fuse_resx ? nullptr : P->tmp_r.p; f.lo_off = P->tmp_h.lo;
-        f.f16 = f16 ? 1 : 0; f.act_mode = f16 ? ACT_PLAIN : u->act_mode;
-        const size_t smem = (round_up(C * (S[0] + 2) * (S[0] + 2), 4) + 10 * C * dp[0]) * sizeof(float);
-        PROF_BEGIN(prof, KC_FIRST, "enc1.conv1 + res (k_conv_first)", (unsigned)R);
-        k_conv_first<<<(unsigned)R, 256, smem, st>>>(f);
-        PROF_END(prof);
-        DTRAJ_LAUNCH_CHECK(); ++nl;
+    for (Launch& l : P->launches) {
+        const float* tb = l.tb_block >= 0 ? trow + u->tb_off[l.tb_block] : nullptr;
+        if (prof) prof->begin(l.cls, l.name, l.grid, l.flops);
+        const int rc = launch_record(l, u, x, x_stride, row_sample, row_variant, tb, per_row, st);
+        if (prof) prof->end();
+        DTRAJ_TRY(rc);
     }
-    size_t ci = 0;
-    auto conv = [&]() -> int {
-        dtraj_plan::ConvOp& op = P->convs[ci++];
-        const float* tb = op.tb_block >= 0 ? trow + u->tb_off[op.tb_block] : nullptr;
-        ++nl;
-        int rc;
-        PROF_BEGIN(prof, KC_CONV, op.name, op.umma ? op.U.grid : 0u, op.flops);
-        if (op.umma) {
-            op.U.conv.L.tbias = tb; op.U.conv.L.row_variant = row_variant; op.U.conv.L.tb_rows = per_row ? 1 : 0;
-            if (op.needs_x) { op.U.conv.L.xraw = x; op.U.conv.L.x_stride = x_stride; op.U.conv.L.row_sample = row_sample; }
-            rc = launch_conv_umma(op.U, st);
-        } else {
-            op.L.tbias = tb; op.L.row_variant = row_variant;
-            rc = launch_conv_simt(op.L, st);
-        }
-        PROF_END(prof);
-        return rc;
-    };
-    auto pool = [&](const dtraj_plan::Buf& in, const dtraj_plan::Buf& out, int So, int cp, int level) -> int {
-        if (P->fuse_pool[level]) return 0;      // emitted by the producing conv's epilogue
-        const int64_t n4 = R * So * So * (cp / 4);
-        PROF_BEGIN(prof, KC_RESAMPLE, "maxpool 2x2");
-        if (f16) k_pool2_h<<<blocks_for(n4 / 2, 256), 256, 0, st>>>((const __half*)in.p, (__half*)out.p, n4 / 2, So, So, cp / 8);
-        else k_pool2<<<blocks_for(n4, 256), 256, 0, st>>>(in.p, out.p, n4, So, So, cp / 4, out.lo, out.lo ? ACT_SPLIT : ACT_PLAIN);
-        PROF_END(prof);
-        DTRAJ_LAUNCH_CHECK(); ++nl;
-        return 0;
-    };
-    auto upsample = [&](const dtraj_plan::Buf& in, const dtraj_plan::Buf& out, int Si, int cp) -> int {
-        const int64_t n4 = R * (2 * Si) * (2 * Si) * (cp / 4);
-        if (n4 >= ((int64_t)1 << 31)) return fail(DTRAJ_EINVAL, "upsample: batch too large for 32-bit indexing");
-        PROF_BEGIN(prof, KC_RESAMPLE, Si == 1 ? "upsample 1->2" : Si == 2 ? "upsample 2->4" : Si == 4 ? "upsample 4->8" : Si == 8 ? "upsample 8->16" : "upsample");
-        Up2Coef cf;
-        const int cp8 = cp / 8;
-        if (f16 && (cp8 & (cp8 - 1)) == 0 && up2_static_ok(Si, &cf)) {
-            int lg_hi = 0, lg_c = 0;
-            while ((1 << lg_hi) < Si) ++lg_hi;
-            while ((1 << lg_c) < cp8) ++lg_c;
-            const int64_t n_blk = R * Si * Si * cp8;
-            DTRAJ_CUDA(launch_ex(k_upsample2_h4, blocks_for(n_blk, 256), 256, 0, st, 1, true, (const __half*)in.p, (__half*)out.p,
-                                 (uint32_t)n_blk, Si, lg_hi, cp8, lg_c, cf));
-        } else if (f16) DTRAJ_CUDA(launch_ex(k_upsample2_h, blocks_for(n4 / 2, 256), 256, 0, st, 1, true, (const __half*)in.p, (__half*)out.p, n4 / 2, Si, Si, cp / 8));
-        else k_upsample2<<<blocks_for(n4, 256), 256, 0, st>>>(in.p, out.p, n4, Si, Si, cp / 4, out.lo,
-                                                             (u->act_mode == ACT_SPLIT && !out.lo) ? ACT_PLAIN : u->act_mode);
-        PROF_END(prof);
-        DTRAJ_LAUNCH_CHECK(); ++nl;
-        return 0;
-    };
-    const dtraj_plan::Buf* pool_in[4] = {&P->tmp_x, &P->x2, &P->x3, &P->x4};
-    const dtraj_plan::Buf* pool_out[4] = {&P->p1, &P->p2, &P->p3, &P->p4};
-    const dtraj_plan::Buf* up[3] = {&P->u3, &P->u2, &P->u1};
-    const int upc[3] = {dp[3], dp[2], dp[1]};
-    for (const dtraj_plan::Op& op : P->seq) {
-        if (op.kind == 0) DTRAJ_TRY(conv());
-        else if (op.kind == 1) DTRAJ_TRY(pool(*pool_in[op.a], *pool_out[op.a], S[op.a + 1], dp[op.a], op.a));
-        else DTRAJ_TRY(upsample(P->tmp_x, *up[op.a], S[4 - op.a], upc[op.a]));
+    return 0;
+}
+
+// dtraj_unet_forward*: (re)build the handle's cached plan for this batch and workspace, run it, expand eps to full resolution
+int unet_forward(dtraj_unet* u, const float* x, int64_t n_rows, int t, const int32_t* row_variant, bool per_row, float* eps,
+                 void* workspace, int64_t workspace_bytes, cudaStream_t st) {
+    if (!u->plan || u->plan->R != n_rows || u->plan->ws != (float*)workspace) {
+        if (u->plan) { delete u->plan; u->plan = nullptr; }
+        DTRAJ_TRY(plan_build(u, n_rows, workspace, workspace_bytes, &u->plan));
     }
-    if (!P->fuse_final) {   // final 1x1 at half resolution (else: dec1.conv2's epilogue)
-        const int64_t npix = R * S[1] * S[1];
-        PROF_BEGIN(prof, KC_RESAMPLE, "final 1x1");
-        k_final1x1<<<blocks_for(npix * 32, 256), 256, 0, st>>>(P->y1.p, u->finw, u->finb, P->elow.p, npix, dp[0], C);
-        PROF_END(prof);
-        DTRAJ_LAUNCH_CHECK(); ++nl;
-    }
-    if (launches) *launches += nl;
+    const int C = u->d.channels, H = u->d.image_size;
+    DTRAJ_TRY(plan_forward(u->plan, x, (int64_t)C * H * H, nullptr, row_variant, t, per_row, st));
+    const int64_t n = n_rows * C * H * H;
+    k_eps_out<<<blocks_for(n, 256), 256, 0, st>>>(u->plan->elow.p, eps, n, C, H, H);
+    DTRAJ_LAUNCH_CHECK();
     return 0;
 }
 
@@ -737,33 +755,13 @@ extern "C" int dtraj_unet_destroy(dtraj_unet* u) {
 extern "C" int dtraj_unet_forward(dtraj_unet* u, const float* x, int64_t n_rows, int32_t t, const int32_t* row_variant,
                                   float* eps, void* workspace, int64_t workspace_bytes, void* stream) {
     if (!u || !x || !eps || !workspace) return fail(DTRAJ_EINVAL, "null argument");
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!u->plan || u->plan->R != n_rows || u->plan->ws != (float*)workspace) {
-        if (u->plan) { delete u->plan; u->plan = nullptr; }
-        DTRAJ_TRY(plan_build(u, n_rows, workspace, workspace_bytes, &u->plan));
-    }
-    const int C = u->d.channels, H = u->d.image_size;
-    DTRAJ_TRY(plan_forward(u->plan, x, (int64_t)C * H * H, nullptr, row_variant, t, st, nullptr));
-    const int64_t n = n_rows * C * H * H;
-    k_eps_out<<<blocks_for(n, 256), 256, 0, st>>>(u->plan->elow.p, eps, n, C, H, H);
-    DTRAJ_LAUNCH_CHECK();
-    return 0;
+    return unet_forward(u, x, n_rows, t, row_variant, false, eps, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int dtraj_unet_forward_rows(dtraj_unet* u, const float* x, int64_t n_rows, const int32_t* row_tv, float* eps,
                                        void* workspace, int64_t workspace_bytes, void* stream) {
     if (!u || !x || !eps || !workspace || !row_tv) return fail(DTRAJ_EINVAL, "null argument");
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!u->plan || u->plan->R != n_rows || u->plan->ws != (float*)workspace) {
-        if (u->plan) { delete u->plan; u->plan = nullptr; }
-        DTRAJ_TRY(plan_build(u, n_rows, workspace, workspace_bytes, &u->plan));
-    }
-    const int C = u->d.channels, H = u->d.image_size;
-    DTRAJ_TRY(plan_forward(u->plan, x, (int64_t)C * H * H, nullptr, row_tv, 0, st, nullptr, nullptr, true));
-    const int64_t n = n_rows * C * H * H;
-    k_eps_out<<<blocks_for(n, 256), 256, 0, st>>>(u->plan->elow.p, eps, n, C, H, H);
-    DTRAJ_LAUNCH_CHECK();
-    return 0;
+    return unet_forward(u, x, n_rows, 0, row_tv, true, eps, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int dtraj_step_fused(int32_t rule, const float* k, const float* eps_u, const float* eps_c, const float* w,
@@ -791,23 +789,27 @@ struct dtraj_sampler {
     dtraj_plan* plan0 = nullptr;    // first step with shared rows (desc.n_rows0 > 0); same workspace
     cudaGraph_t graph = nullptr;
     cudaGraphExec_t exec = nullptr;
-    int64_t launches = 0;
 };
 
 namespace {
 
-int sampler_enqueue(dtraj_sampler* s, cudaStream_t st, int64_t* launches, Profiler* prof = nullptr) {
+// a per-forward quantity of the plans summed over the loop: step 0 runs the shared-row plan when there is one
+template <class F> auto per_loop(const dtraj_sampler* s, F per_forward) -> decltype(per_forward(s->plan)) {
+    const int nu = s->d.n_updates;
+    return nu > 0 ? per_forward(s->plan0 ? s->plan0 : s->plan) + per_forward(s->plan) * (nu - 1) : 0;
+}
+
+int sampler_enqueue(dtraj_sampler* s, cudaStream_t st, Profiler* prof = nullptr) {
     const dtraj_sampler_desc& d = s->d;
     const int C = s->u->d.channels, H = s->u->d.image_size;
     const int64_t D = (int64_t)C * H * H, fs = (int64_t)d.n_frames * D;
-    int64_t nl = 0;
     for (int k = 0; k < d.n_updates; ++k) {
         if (prof) prof->step = k;
         const float* xin = d.traj + (int64_t)k * D;
         const bool first = k == 0 && s->plan0 != nullptr;            // shared rows: every sample of a group still has x_T
         dtraj_plan* P = first ? s->plan0 : s->plan;
         DTRAJ_TRY(plan_forward(P, xin, fs, first ? d.row_sample0 : d.row_sample, first ? d.row_variant0 : d.row_variant,
-                               s->ts[k], st, &nl, prof));
+                               s->ts[k], false, st, prof));
         StepParams p;
         p.rule = d.rule; p.k0 = s->coef[3 * k]; p.k1 = s->coef[3 * k + 1]; p.k2 = s->coef[3 * k + 2];
         p.elow = P->elow.p; p.sample_row_u = first ? d.sample_row_u0 : d.sample_row_u;
@@ -816,21 +818,21 @@ int sampler_enqueue(dtraj_sampler* s, cudaStream_t st, int64_t* launches, Profil
         p.z_index = d.z_index ? d.z_index + (int64_t)k * d.n_samples : nullptr;
         p.x_in = xin; p.x_out = d.traj + (int64_t)(k + 1) * D; p.frame_stride = fs;
         p.B = d.n_samples; p.C = C; p.H = H; p.W = H;
-        const int64_t nthr = (int64_t)d.n_samples * C * H * (H / 4);
-        PROF_BEGIN(prof, KC_STEP, "k_step (CFG + update + store)");
-        DTRAJ_CUDA(launch_ex(k_step, blocks_for(nthr, 256), 256, 0, st, 1, s->u->d.precision == DTRAJ_PREC_F16, p));
-        PROF_END(prof);
-        DTRAJ_LAUNCH_CHECK(); ++nl;
+        const unsigned grid = blocks_for((int64_t)d.n_samples * C * H * (H / 4), 256);
+        if (prof) prof->begin(KC_STEP, "k_step (CFG + update + store)", grid, 0.0);
+        DTRAJ_CUDA(launch_ex(k_step, grid, 256, 0, st, 1, s->u->d.precision == DTRAJ_PREC_F16, p));
+        if (prof) prof->end();
+        DTRAJ_LAUNCH_CHECK();
     }
     if (d.copy_last) {
         const int64_t k = d.n_updates;
-        PROF_BEGIN(prof, KC_STEP, "k_copy_frame");
-        DTRAJ_CUDA(launch_ex(k_copy_frame, blocks_for((int64_t)d.n_samples * (D / 4), 256), 256, 0, st, 1, s->u->d.precision == DTRAJ_PREC_F16,
-                             (const float*)(d.traj + k * D), d.traj + (k + 1) * D, fs, d.n_samples, (int)(D / 4)));
-        PROF_END(prof);
-        DTRAJ_LAUNCH_CHECK(); ++nl;
+        const unsigned grid = blocks_for((int64_t)d.n_samples * (D / 4), 256);
+        if (prof) prof->begin(KC_STEP, "k_copy_frame", grid, 0.0);
+        DTRAJ_CUDA(launch_ex(k_copy_frame, grid, 256, 0, st, 1, s->u->d.precision == DTRAJ_PREC_F16, (const float*)(d.traj + k * D),
+                             d.traj + (k + 1) * D, fs, d.n_samples, (int)(D / 4)));
+        if (prof) prof->end();
+        DTRAJ_LAUNCH_CHECK();
     }
-    if (launches) *launches = nl;
     return 0;
 }
 
@@ -882,7 +884,7 @@ extern "C" int dtraj_sampler_create(dtraj_unet* u, const dtraj_sampler_desc* d, 
         if (ce != cudaSuccess) { dtraj_sampler_destroy(s); return fail(DTRAJ_ECUDA, "stream create -> %s", cudaGetErrorString(ce)); }
         ce = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
         if (ce == cudaSuccess) {
-            rc = sampler_enqueue(s, cs, &s->launches);
+            rc = sampler_enqueue(s, cs);
             cudaError_t ce2 = cudaStreamEndCapture(cs, &s->graph);
             if (rc == 0 && ce2 != cudaSuccess) rc = fail(DTRAJ_ECUDA, "graph capture -> %s", cudaGetErrorString(ce2));
             if (rc == 0) {
@@ -892,11 +894,6 @@ extern "C" int dtraj_sampler_create(dtraj_unet* u, const dtraj_sampler_desc* d, 
         } else rc = fail(DTRAJ_ECUDA, "begin capture -> %s", cudaGetErrorString(ce));
         cudaStreamDestroy(cs);
         if (rc) { dtraj_sampler_destroy(s); return rc; }
-    } else {
-        // dry count of launches: enc1 stage + the plan's ops (fused pools launch nothing) + final 1x1 + fused step
-        int64_t per = 1 + (s->plan->fuse_final ? 0 : 1) + 1;
-        for (const dtraj_plan::Op& op : s->plan->seq) per += (op.kind == 1 && s->plan->fuse_pool[op.a]) ? 0 : 1;
-        s->launches = (int64_t)d->n_updates * per + (d->copy_last ? 1 : 0);
     }
     *out = s;
     return 0;
@@ -906,27 +903,45 @@ extern "C" int dtraj_sampler_run(dtraj_sampler* s, void* stream) {
     if (!s) return fail(DTRAJ_EINVAL, "null sampler");
     cudaStream_t st = (cudaStream_t)stream;
     if (s->exec) { DTRAJ_CUDA(cudaGraphLaunch(s->exec, st)); return 0; }
-    return sampler_enqueue(s, st, nullptr);
+    return sampler_enqueue(s, st);
 }
 
-extern "C" int64_t dtraj_sampler_launches(const dtraj_sampler* s) { return s ? s->launches : -1; }
+// per update one forward and one k_step, then the frame copy
+extern "C" int64_t dtraj_sampler_launches(const dtraj_sampler* s) {
+    if (!s) return -1;
+    return per_loop(s, [](const dtraj_plan* P) { return (int64_t)P->launches.size(); }) + s->d.n_updates + (s->d.copy_last ? 1 : 0);
+}
 
 namespace {
 
 // executed conv flops of a whole loop (real channels, evaluated taps): [0] generic convs, [1] the fused enc1 kernel's conv2
 void sampler_flops(const dtraj_sampler* s, double* out2) {
-    auto plan_flops = [&](const dtraj_plan* P, double* conv, double* e1) {
-        double f = 0.0;
-        for (auto& op : P->convs) f += op.flops;
-        *conv = f;
-        *e1 = P->fuse_enc1 ? (s->u->d.precision == DTRAJ_PREC_F16 ? P->enc1h.flops : P->enc1.flops) : 0.0;
+    auto flops_of = [&](int cls) {
+        return per_loop(s, [cls](const dtraj_plan* P) {
+            double f = 0.0;
+            for (const Launch& l : P->launches)
+                if (l.cls == cls) f += l.flops;
+            return f;
+        });
     };
-    double fc = 0.0, fe = 0.0, fc0 = 0.0, fe0 = 0.0;
-    plan_flops(s->plan, &fc, &fe);
-    if (s->plan0) plan_flops(s->plan0, &fc0, &fe0); else { fc0 = fc; fe0 = fe; }
-    const int nu = s->d.n_updates;
-    out2[0] = nu > 0 ? fc0 + fc * (nu - 1) : 0.0;       // the first step runs the shared-row plan
-    out2[1] = nu > 0 ? fe0 + fe * (nu - 1) : 0.0;
+    out2[0] = flops_of(KC_CONV);
+    out2[1] = flops_of(KC_ENC1);
+}
+
+// Runs the loop once, un-captured, with an event pair around every launch on `st`; appends the records of the launches
+// that completed, with their device milliseconds, to `out`.  Synchronises the stream.
+int profile_run(dtraj_sampler* s, cudaStream_t st, std::vector<Profiler::Rec>* out) {
+    Profiler prof;
+    prof.st = st;
+    const int rc = sampler_enqueue(s, st, &prof);
+    const cudaError_t ce = cudaStreamSynchronize(st);
+    for (Profiler::Rec& r : prof.recs) {
+        if (rc == 0 && ce == cudaSuccess && cudaEventElapsedTime(&r.ms, r.a, r.b) == cudaSuccess) out->push_back(r);
+        cudaEventDestroy(r.a); cudaEventDestroy(r.b);
+    }
+    if (rc) return rc;
+    if (ce != cudaSuccess) return fail(DTRAJ_ECUDA, "profile -> %s", cudaGetErrorString(ce));
+    return 0;
 }
 
 }  // namespace
@@ -939,43 +954,25 @@ extern "C" int dtraj_sampler_flops(const dtraj_sampler* s, double* conv_flops2) 
 
 extern "C" int dtraj_sampler_profile(dtraj_sampler* s, void* stream, double* class_ms, int64_t* class_launches, double* conv_flops) {
     if (!s || !class_ms || !class_launches || !conv_flops) return fail(DTRAJ_EINVAL, "profile: null argument");
-    Profiler prof;
-    prof.st = (cudaStream_t)stream;
-    int rc = sampler_enqueue(s, prof.st, nullptr, &prof);
-    cudaError_t ce = cudaStreamSynchronize(prof.st);
+    std::vector<Profiler::Rec> recs;
+    const int rc = profile_run(s, (cudaStream_t)stream, &recs);
     for (int c = 0; c < KC_COUNT; ++c) { class_ms[c] = 0.0; class_launches[c] = 0; }
-    for (auto& r : prof.recs) {
-        float ms = 0.f;
-        if (rc == 0 && ce == cudaSuccess && cudaEventElapsedTime(&ms, r.a, r.b) == cudaSuccess) {
-            class_ms[r.cls] += ms;
-            class_launches[r.cls] += 1;
-        }
-        cudaEventDestroy(r.a); cudaEventDestroy(r.b);
-    }
+    for (const Profiler::Rec& r : recs) { class_ms[r.cls] += r.ms; class_launches[r.cls] += 1; }
     sampler_flops(s, conv_flops);
-    if (rc) return rc;
-    if (ce != cudaSuccess) return fail(DTRAJ_ECUDA, "profile -> %s", cudaGetErrorString(ce));
-    return 0;
+    return rc;
 }
 
 extern "C" int dtraj_sampler_profile_text(dtraj_sampler* s, void* stream, int32_t step, char* buf, int64_t buf_len) {
     if (!s || !buf || buf_len < 64) return fail(DTRAJ_EINVAL, "profile_text: bad argument");
     if (step < 0 || step >= s->d.n_updates) return fail(DTRAJ_EINVAL, "profile_text: step %d outside 0..%d", step, s->d.n_updates - 1);
-    Profiler prof;
-    prof.st = (cudaStream_t)stream;
-    int rc = sampler_enqueue(s, prof.st, nullptr, &prof);
-    cudaError_t ce = cudaStreamSynchronize(prof.st);
+    std::vector<Profiler::Rec> recs;
+    const int rc = profile_run(s, (cudaStream_t)stream, &recs);
     int64_t off = 0;
     buf[0] = 0;
-    for (auto& r : prof.recs) {
-        float ms = 0.f;
-        if (rc == 0 && ce == cudaSuccess && r.step == step && cudaEventElapsedTime(&ms, r.a, r.b) == cudaSuccess && off + 128 < buf_len)
-            off += snprintf(buf + off, (size_t)(buf_len - off), "%s\t%u\t%.2f\t%.6g\n", r.name, r.grid, ms * 1e3, r.flops);
-        cudaEventDestroy(r.a); cudaEventDestroy(r.b);
-    }
-    if (rc) return rc;
-    if (ce != cudaSuccess) return fail(DTRAJ_ECUDA, "profile_text -> %s", cudaGetErrorString(ce));
-    return 0;
+    for (const Profiler::Rec& r : recs)
+        if (r.step == step && off + 128 < buf_len)
+            off += snprintf(buf + off, (size_t)(buf_len - off), "%s\t%u\t%.2f\t%.6g\n", r.name, r.grid, r.ms * 1e3, r.flops);
+    return rc;
 }
 
 // ======================================================================================

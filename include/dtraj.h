@@ -190,7 +190,8 @@ int64_t dtraj_sampler_launches(const dtraj_sampler* s);
  * every launch on `stream`, and returns the summed device time (ms) and launch count per kernel class
  *   [0] generic convolutions (tcgen05 implicit GEMM, or the CUDA-core kernel in DTRAJ_PREC_FP32)
  *   [1] first convolution (Cin <= 4)   [2] max-pool / upsample / final 1x1   [3] fused step / frame copy
- *   [4] fused enc1 block (conv1 on CUDA cores into shared memory + conv2 by tap views + pool)
+ *   [4] fused enc1 block (conv1 into shared memory + conv2 by tap views + pool; conv1 runs on the tensor cores in
+ *       DTRAJ_PREC_F16, on the CUDA cores in DTRAJ_PREC_TF32)
  * plus the algorithmic tensor-core flops of class 0 (conv_flops2[0]) and of class 4 (conv_flops2[1]): sum over
  * layers and steps of 2 * M * Cout * Cin * taps with REAL (unpadded) channel counts and the taps actually
  * evaluated.  Synchronises the stream.
