@@ -80,10 +80,19 @@ struct UmmaConv {
     int f16;                   // 1: DTRAJ_PREC_F16 -- fp16 feature maps / weights (64 channels per 128-byte K block), kind::f16 MMAs
     int halo;                  // HALO mode (fp16, 3x3): a tile's pixels arrive ONCE per 64-channel chunk as a halo box, the nine taps are
                                //    descriptor views of it.  1: 8x8 maps, a tile = two images, halos [10 rows][2 images][10 pixels] through
-                               //    the permuted dimensions {c, x, image, y};  2: 16x16 maps, a tile = the left or right half (16 rows x 8
-                               //    columns) of one image, halo [18 rows][10 pixels] through the standard dimensions {c, x, y, image}
+                               //    the permuted dimensions {c, x, image, y};  2: 16x16 and 32x32 maps, a tile = 16 rows x 8 columns of one
+                               //    image, halo [18 rows][10 pixels] through the standard dimensions {c, x, y, image}
     int n_hb;                  // halo ring depth
+    int hlg_x, hlg_t;          // halo mode 2: log2 of the 8-column groups per image (1 at 16x16, 2 at 32x32) and of the tiles per image
+                               //    (1, 3): tile t covers image t >> hlg_t, columns from (t & (2^hlg_x - 1)) * 8, rows from the band above
 };
+
+// halo mode 2: image, first row and first column of tile `t`
+__device__ __forceinline__ void halo2_tile(const UmmaConv& p, int t, int& img, int& y0, int& x0) {
+    img = t >> p.hlg_t;
+    x0 = (t & ((1 << p.hlg_x) - 1)) * 8;
+    y0 = ((t & ((1 << p.hlg_t) - 1)) >> p.hlg_x) * 16;
+}
 
 constexpr uint32_t kHaloBytes = 26624;     // 200 halo pixels x 128 B, rounded up to 1024
 constexpr uint32_t kHaloTx = 200 * 128;    // bytes one halo box delivers
@@ -428,8 +437,9 @@ k_conv_umma_t(const __grid_constant__ UmmaMaps maps, const UmmaConv p) {
                     uint32_t fb = hfull0 + 8u * hb;
                     if constexpr (kPair) fb = ptx::map_to_cta(fb, 0);
                     if (!kPair || crank == 0) ptx::mbar_expect_tx(hfull0 + 8u * hb, bytes * (kPair ? 2u : 1u));
-                    // mode 1: dims {c, x, image, y}, two images from 2 * tile;  mode 2: dims {c, x, y, image}, columns from (tile & 1) * 8
-                    const int k1 = p.halo == 1 ? xy0 : (tile & 1) * 8 + xy0, k2 = p.halo == 1 ? 2 * tile : xy0, k3 = p.halo == 1 ? xy0 : tile >> 1;
+                    // mode 1: dims {c, x, image, y}, two images from 2 * tile;  mode 2: dims {c, x, y, image}, 16 x 8 pixels from (y0, x0)
+                    int k1 = xy0, k2 = 2 * tile, k3 = xy0;
+                    if (p.halo == 2) { int ty, tx; halo2_tile(p, tile, k3, ty, tx); k1 = tx + xy0; k2 = ty + xy0; }
                     if constexpr (kPair) ptx::tma_load_4d_2sm(halo_base + hb * kHaloBytes, am, fb, c0, k1, k2, k3);
                     else ptx::tma_load_4d(halo_base + hb * kHaloBytes, am, fb, c0, k1, k2, k3);
                     if (++hb == p.n_hb) { hb = 0; hph ^= 1u; }
@@ -757,9 +767,10 @@ k_conv_umma_t(const __grid_constant__ UmmaMaps maps, const UmmaConv p) {
             const int tile = work / p.n_split, n0 = (work % p.n_split) * ncols;
             const int64_t m_warp = (int64_t)tile * 128 + q * 32;
             const int row = (int)m_warp;
-            const int hx0 = p.halo == 2 ? (tile & 1) * 8 : 0;       // halo mode 2: first column of the tile's half image
-            // coordinates of this warp's 32-row box in the 4-d output / residual maps (halo modes)
-            int hk1 = p.halo == 1 ? 0 : hx0, hk2 = p.halo == 1 ? 2 * tile : 4 * q, hk3 = p.halo == 1 ? 2 * q : (tile >> 1);
+            // coordinates of this warp's 32-row box in the 4-d output / residual maps (halo modes; mode 2: the tile's first
+            // column, its first row + 4q, its image)
+            int hk1 = 0, hk2 = 2 * tile, hk3 = 2 * q;
+            if (p.halo == 2) { halo2_tile(p, tile, hk3, hk2, hk1); hk2 += 4 * q; }
             int pm_pos = 0, pm_img0 = 0;
             if (p.posm) {                                           // box {32 ch, 1, 1, 32 images} at (x, y, first image of the warp)
                 pm_pos = tile / p.nblk_img;
@@ -793,11 +804,11 @@ k_conv_umma_t(const __grid_constant__ UmmaMaps maps, const UmmaConv p) {
                 valid = (int64_t)img * 64 < p.L.M;
                 m = (int64_t)img * 64 + (r >> 4) * 8 + (r & 7);
                 if (!valid) img = 0;
-            } else if (p.halo == 2) {                                // rows ordered (y, x): y = r >> 3 of 16, x = x0 + (r & 7)
+            } else if (p.halo == 2) {                                // rows ordered (y, x): y = y0 + (r >> 3), x = x0 + (r & 7)
                 const int r = q * 32 + lane;
-                img = tile >> 1;
-                valid = (int64_t)img * 256 < p.L.M;
-                m = (int64_t)img * 256 + (r >> 3) * 16 + hx0 + (r & 7);
+                img = hk3;
+                valid = ((int64_t)img << p.log2_hw) < p.L.M;
+                m = ((int64_t)img << p.log2_hw) + (hk2 + (lane >> 3)) * p.L.W + hk1 + (r & 7);
                 if (!valid) img = 0;
             } else if (p.posm) {                                     // rows = images at one position
                 img = pm_img0 + lane;
@@ -954,8 +965,8 @@ k_conv_umma_t(const __grid_constant__ UmmaMaps maps, const UmmaConv p) {
                     } else if (p.halo == 2) {                            // warp rows = (y in 4q .. 4q+3, x in x0 .. x0+7): 2 x 4 windows
                         const int wy = pr >> 2, wx = pr & 3;
                         r00 = wy * 16 + 2 * wx; rdn = 8;
-                        prow = ((int64_t)(tile >> 1) * 8 + 2 * q + wy) * 8 + (hx0 >> 1) + wx;
-                        pvalid = (int64_t)(tile >> 1) * 256 < p.L.M;
+                        prow = ((int64_t)hk3 * (W >> 1) + (hk2 >> 1) + wy) * (W >> 1) + (hk1 >> 1) + wx;
+                        pvalid = ((int64_t)hk3 << p.log2_hw) < p.L.M;
                     }
                     if (pvalid) {
                         const uint32_t jj = (uint32_t)(lane & 3);
@@ -1389,11 +1400,16 @@ inline bool umma_posm_applies(int H, int64_t n_img) {
 }
 
 // `w_rows` = rows of the packed weight matrix (hi planes then, for 3 passes, lo planes)
+// `form` (dtraj_bench_conv's A/B experiments; the forward plan passes 0): 0 = the form and shared-memory split chosen below;
+// kUmmaGeneric = the generic [image][y][x] tiles even where a halo form exists; kUmmaSplit | n_hb << 4 | epi_bufs = the halo form
+// with that many halo slots and epilogue buffers per warp, the rest of the shared memory as weight stages (at most 16)
+constexpr int kUmmaGeneric = 1, kUmmaSplit = 0x100;
 inline int build_umma_launch(UmmaLaunch* U, const ConvLayer& L, int npass, const float* wpk, int64_t w_rows,
-                             const float* rwpk = nullptr, int64_t rw_rows = 0) {
+                             const float* rwpk = nullptr, int64_t rw_rows = 0, int form = 0) {
     memset(U, 0, sizeof(*U));
     const int HW = L.H * L.W;
-    if (L.W > 32 || L.H != L.W || (HW & (HW - 1)) != 0)
+    // (a tile is 128 / W whole image rows: 2 at 64x64, the largest map of a supported model)
+    if (L.W > 64 || L.H != L.W || (HW & (HW - 1)) != 0)
         return fail(DTRAJ_EINVAL, "umma conv: unsupported spatial size %dx%d", L.H, L.W);
     const int f16 = L.f16 ? 1 : 0, kch = f16 ? 64 : 32;     // channels per 128-byte K block
     // channel counts are padded to 32 in every mode; in fp16 mode a K block carries 64 channels, so a source padded to an odd
@@ -1478,9 +1494,11 @@ inline int build_umma_launch(UmmaLaunch* U, const ConvLayer& L, int npass, const
     // (N <= 128: <= 256 cycles per K block) and the stage stays small enough to keep >= 3 stages in flight
     const int n_stage_rows = c.pair ? n_rows / 2 : n_rows;
     c.kbs = (n_stage_rows <= (c.pair ? 64 : 128) && c.r_nch0 % 2 == 0 && (c.r_nch - c.r_nch0) % 2 == 0 && c.nch0 % 2 == 0 && (c.nch - c.nch0) % 2 == 0) ? 2 : 1;
-    // halo mode (fp16, 8x8 maps, 3x3, no identity residual): two images per tile, pixels through the halo ring
-    c.halo = (f16 && L.ntaps == 9 && !(L.flags & CONV_RESX) && c.n_split == 1 && L.act_mode != ACT_SPLIT)
-                 ? (L.H == 8 && L.W == 8 ? 1 : (L.H == 16 && L.W == 16 ? 2 : 0)) : 0;
+    // halo mode (fp16, 8x8 / 16x16 / 32x32 maps, 3x3, no identity residual): pixels through the halo ring
+    c.halo = (form != kUmmaGeneric && f16 && L.ntaps == 9 && !(L.flags & CONV_RESX) && c.n_split == 1 && L.act_mode != ACT_SPLIT)
+                 ? (L.H == 8 && L.W == 8 ? 1 : ((L.H == 16 || L.H == 32) && L.W == L.H ? 2 : 0)) : 0;
+    c.hlg_x = L.W == 32 ? 2 : 1;
+    c.hlg_t = L.W == 32 ? 3 : 1;
     if (c.posm && (c.half_mask || c.r_half_mask || c.n_split > 1)) c.kbs = 1;   // (position-major tiles: two K blocks per stage where every chunk is a full one)
     c.n_hb = 0;
     // (halo mode: kbs = weight tiles (taps) per stage -- all nine where a tile is at most 4 KB, three where it is 8 KB, i.e. where four
@@ -1498,6 +1516,8 @@ inline int build_umma_launch(UmmaLaunch* U, const ConvLayer& L, int npass, const
     // trade loses on the 8-chunk dec1.conv1 and on 8 KB stages, same file)
     const bool halo_short = c.halo && !(L.flags & CONV_RESACC) && c.nch <= 2 && n_stage_rows * 128 >= 16384;
     if (halo_short) c.n_hb = 2;
+    const bool split_set = c.halo && (form & kUmmaSplit);
+    if (split_set) c.n_hb = (form >> 4) & 15;
     if (c.n_hb > 4) return fail(DTRAJ_EINVAL, "umma conv: the kernel has four halo-ring barriers");
     const size_t stage = c.halo ? (size_t)c.kbs * n_stage_rows * 128 : (size_t)c.kbs * (kATileBytes + (size_t)n_stage_rows * 128);
     const size_t cst_bytes = (size_t)(5 + ((L.flags & CONV_FINAL) ? 4 : 0)) * L.coutp * 4;     // staged per-channel constants
@@ -1507,11 +1527,17 @@ inline int build_umma_launch(UmmaLaunch* U, const ConvLayer& L, int npass, const
     c.epi_bufs = 2;
     c.epi_kind = f16 ? epi_kind_of(L.flags) : 0;
     if (!c.halo && nkb_all >= 16 && stages_for(1) > stages_for(2) && stages_for(2) < 8) c.epi_bufs = 1;
-    if ((halo_res || halo_short) && stages_for(2) < 16) c.epi_bufs = 1;
+    // (at 32x32 the short conv1 keeps its double-buffered epilogue ring: enc2.conv1 of 3x64x64 models at 7680 rows, teacher 2760 -> 2704 us,
+    //  sf 0.5 1549 -> 1468 us with two halo slots; the other 32x32 layers are best with the 16x16 rules, profiles/r03b_halo_split_ab.txt)
+    if ((halo_res || (halo_short && L.W != 32)) && stages_for(2) < 16) c.epi_bufs = 1;
+    if (split_set) {
+        c.epi_bufs = form & 15;
+        if (c.n_hb < 1 || c.epi_bufs < 1 || c.epi_bufs > kEpiBufsMax) return fail(DTRAJ_EINVAL, "umma conv: bad shared-memory split 0x%x", form);
+    }
     int stages = stages_for(c.epi_bufs);
     if (stages < 2) return fail(DTRAJ_EINVAL, "umma conv: operand ring does not fit");
     if (stages > 16) stages = 16;
-    if (c.halo && !halo_res && stages > 12) stages = 12;      // (dec1.conv1: 484 us with 10-12 weight stages, 495 with 14, 510 with 8, 550 with 6)
+    if (c.halo && !halo_res && !split_set && stages > 12) stages = 12;      // (dec1.conv1: 484 us with 10-12 weight stages, 495 with 14, 510 with 8, 550 with 6)
     c.stages = stages;
     U->smem = misc + (size_t)kEpiWarps * c.epi_bufs * epi_buf_bytes + stages * stage;
     U->grid = (unsigned)(c.n_work < kNumSMs ? c.n_work : kNumSMs);
@@ -1561,18 +1587,18 @@ inline int build_umma_launch(UmmaLaunch* U, const ConvLayer& L, int npass, const
         if (L.flags & CONV_RESID) DTRAJ_TRY(mapp(&U->maps.res, L.resid, L.coutp, 32, 32, f16 != 0));
         return 0;
     }
-    if (c.halo == 2) {  // 16x16 maps: standard dimensions {c, x, y, image}; halo box 10 x 18, residual-conv box 8 x 16, output / residual box 8 x 4
+    if (c.halo == 2) {  // 16x16 / 32x32 maps: standard dimensions {c, x, y, image}; halo box 10 x 18, residual-conv box 8 x 16, output / residual box 8 x 4
         auto map4 = [&](CUtensorMap* m, const float* base, int cp, int bc, int bx, int by, bool sw64) -> int {
             PFN_encodeTiled enc = get_encode_tiled();
             if (!enc) return fail(DTRAJ_ECUDA, "cuTensorMapEncodeTiled not available");
-            cuuint64_t dims[4] = {(cuuint64_t)cp, 16, 16, (cuuint64_t)n_img};
-            cuuint64_t strides[3] = {(cuuint64_t)cp * 2, (cuuint64_t)16 * cp * 2, (cuuint64_t)256 * cp * 2};
+            cuuint64_t dims[4] = {(cuuint64_t)cp, (cuuint64_t)L.W, (cuuint64_t)L.H, (cuuint64_t)n_img};
+            cuuint64_t strides[3] = {(cuuint64_t)cp * 2, (cuuint64_t)L.W * cp * 2, (cuuint64_t)HW * cp * 2};
             cuuint32_t box[4] = {(cuuint32_t)bc, (cuuint32_t)bx, (cuuint32_t)by, 1};
             cuuint32_t es[4] = {1, 1, 1, 1};
             CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, (void*)base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                              sw64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) return fail(DTRAJ_ECUDA, "cuTensorMapEncodeTiled(16x16 halo map cp=%d n=%lld) -> %d", cp, (long long)n_img, (int)r);
+            if (r != CUDA_SUCCESS) return fail(DTRAJ_ECUDA, "cuTensorMapEncodeTiled(%dx%d halo map cp=%d n=%lld) -> %d", L.H, L.W, cp, (long long)n_img, (int)r);
             return 0;
         };
         DTRAJ_TRY(map4(&U->maps.a[0], L.src0, L.c0p, 64, 10, 18, false));

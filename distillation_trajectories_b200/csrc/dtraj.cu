@@ -168,6 +168,11 @@ void pack_conv(Arena* A, size_t* w_off, size_t* b_off, PackedConv* pc, const flo
     pc->c0 = c0; pc->c1 = c1; pc->cout = cout;
 }
 
+// dynamic shared memory of k_conv_first: the zero-padded C x (H+2) x (H+2) input, then 9C + C rows of coutp weights
+inline size_t first_conv_smem(int C, int H, int coutp) {
+    return (size_t)(round_up(C * (H + 2) * (H + 2), 4) + 10 * C * coutp) * sizeof(float);
+}
+
 }  // namespace
 
 extern "C" const char* dtraj_last_error(void) { return err_buf(); }
@@ -180,7 +185,7 @@ extern "C" int dtraj_unet_create(const dtraj_unet_desc* desc, const char* const*
     if (!desc || !out || !names || !tensors || !numel) return fail(DTRAJ_EINVAL, "null argument");
     const int C = desc->channels, H = desc->image_size, temb = desc->temb_dim, T = desc->n_timesteps;
     if (C < 1 || C > 4) return fail(DTRAJ_EINVAL, "channels=%d unsupported (1..4)", C);
-    if (H < 16 || H > 32 || (H % 16) != 0) return fail(DTRAJ_EINVAL, "image_size=%d unsupported (16 or 32)", H);
+    if (H != 16 && H != 32 && H != 64) return fail(DTRAJ_EINVAL, "image_size=%d unsupported (16, 32 or 64)", H);
     if (temb < 2 || temb > 1024 || T < 1) return fail(DTRAJ_EINVAL, "bad temb_dim/n_timesteps");
     if (desc->precision < 0 || desc->precision > 3) return fail(DTRAJ_EINVAL, "bad precision");
     for (int i = 0; i < 4; ++i)
@@ -331,6 +336,11 @@ extern "C" int dtraj_unet_create(const dtraj_unet_desc* desc, const char* const*
     ce = cudaGetLastError();
     if (ce == cudaSuccess) ce = cudaDeviceSynchronize();
     if (ce != cudaSuccess) { dtraj_unet_destroy(u); return fail(DTRAJ_ECUDA, "time table kernel -> %s", cudaGetErrorString(ce)); }
+    // k_conv_first stages the padded C x (H+2)^2 input and its weights in shared memory.  The attribute belongs to the kernel, not to
+    // this model, so it is set to what the largest supported model needs (4 x 64 x 64, 256 channels: 108 KB): a narrower model
+    // packed later must not lower it below what an earlier, wider one launches with.
+    ce = cudaFuncSetAttribute(k_conv_first, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)first_conv_smem(4, 64, 256));
+    if (ce != cudaSuccess) { dtraj_unet_destroy(u); return fail(DTRAJ_ECUDA, "smem attribute (k_conv_first) -> %s", cudaGetErrorString(ce)); }
     if (desc->precision != DTRAJ_PREC_FP32) {
         ce = umma_set_smem_attr();
         if (ce == cudaSuccess) ce = enc1_set_smem_attr();
@@ -612,7 +622,7 @@ int plan_build(const dtraj_unet* u, int64_t R, void* ws, int64_t ws_bytes, dtraj
         f.w3 = u->fw3; f.b3 = u->fb3; f.w1 = u->fw1; f.b1 = u->fb1; f.tb_var_stride = u->tb_stride;
         f.h = P->tmp_h.p; f.r = fuse_resx ? nullptr : P->tmp_r.p; f.lo_off = P->tmp_h.lo;
         f.f16 = f16 ? 1 : 0; f.act_mode = f16 ? ACT_PLAIN : u->act_mode;
-        l.first_smem = (round_up(C * (S[0] + 2) * (S[0] + 2), 4) + 10 * C * dp[0]) * sizeof(float);
+        l.first_smem = first_conv_smem(C, S[0], dp[0]);
         l.tb_block = 0;
         Tail t = tail_for(0);
         t.resx = fuse_resx;
@@ -1112,20 +1122,27 @@ extern "C" unsigned int dtraj_debug_umma_error(void) {
     return v;
 }
 
-// Kernel-only timing of one conv layer shape (tools/conv_bench.py): device buffers are allocated and
-// zero-filled here, `iters` launches are timed with one event pair.  `debug` must be 0.
+// Kernel-only timing of one conv layer shape (tools/conv_bench.py, tools/bench_image64.py): device buffers are allocated and
+// zero-filled here, `iters` launches are timed with one event pair.  `debug`: 0 = the form and shared-memory split the forward plan
+// uses, 2 = the generic [image][y][x] tiles where that form is a halo form, 0x100 | n_hb << 4 | epi_bufs = the halo form with that
+// shared-memory split (A/B experiments); other values are refused.  flags & CONV_RESACC: x1 (c1 channels) feeds a fused 1x1
+// residual conv instead of the main conv's K loop.
 extern "C" int dtraj_bench_conv(int32_t precision, int32_t c0, int32_t c1, int32_t cout, int64_t n, int32_t H, int32_t ksize,
                                 int32_t flags, int32_t iters, int32_t debug, float* ms_out) {
-    if (debug) return fail(DTRAJ_EINVAL, "bench_conv: the operand knock-out experiments (profiles/r01f_conv_knockout.txt) were removed from the kernels");
+    if (debug != 0 && debug != 2 && !(debug & kUmmaSplit))
+        return fail(DTRAJ_EINVAL, "bench_conv: the operand knock-out experiments (profiles/r01f_conv_knockout.txt) were removed from the kernels");
+    const bool resacc = (flags & CONV_RESACC) != 0;
     const int cpad = kCPad;
     const int c0p = round_up(c0, cpad), c1p = c1 ? round_up(c1, cpad) : 0, coutp = round_up(cout, cpad);
     const int64_t M = n * H * H;
-    std::vector<float> w((size_t)cout * (c0 + c1) * ksize * ksize, 0.01f);
+    const int cm1 = resacc ? 0 : c1;                  // second source of the main conv
+    std::vector<float> w((size_t)cout * (c0 + cm1) * ksize * ksize, 0.01f), wr((size_t)cout * (c1 ? c1 : 1), 0.01f);
     std::vector<double> shift(cout, 0.0);
     Arena A;
-    PackedConv pc;
-    size_t wo, bo;
-    pack_conv(&A, &wo, &bo, &pc, w.data(), cout, c0, c1, ksize, ksize == 3 && H == 1, nullptr, shift.data(), precision);
+    PackedConv pc, pr;
+    size_t wo, bo, wro = 0, bro = 0;
+    pack_conv(&A, &wo, &bo, &pc, w.data(), cout, c0, cm1, ksize, ksize == 3 && H == 1, nullptr, shift.data(), precision);
+    if (resacc) pack_conv(&A, &wro, &bro, &pr, wr.data(), cout, c1, 0, 1, false, nullptr, shift.data(), precision);
     float *dev = nullptr, *x0 = nullptr, *x1 = nullptr, *res = nullptr, *out = nullptr;
     const int planes = precision == DTRAJ_PREC_TF32X3 ? 2 : 1;
     DTRAJ_CUDA(cudaMalloc(&dev, A.h.size() * sizeof(float)));
@@ -1139,10 +1156,11 @@ extern "C" int dtraj_bench_conv(int32_t precision, int32_t c0, int32_t c1, int32
     ConvLayer L;
     memset(&L, 0, sizeof(L));
     L.src0 = x0; L.src0_lo = x0 + (size_t)M * c0p; L.c0p = c0p;
-    L.src1 = x1; L.src1_lo = x1 ? x1 + (size_t)M * c1p : nullptr; L.c1p = c1p;
+    if (resacc) { L.rsrc0 = x1; L.rc0p = pr.c0p; L.rbias = dev + bro; }
+    else { L.src1 = x1; L.src1_lo = x1 ? x1 + (size_t)M * c1p : nullptr; L.c1p = c1p; }
     L.H = H; L.W = H; L.M = M; L.ntaps = pc.ntaps; L.wpk = dev + wo; L.bias = dev + bo; L.coutp = coutp;
     L.resid = (flags & 4) ? res : nullptr; L.out = out; L.lo_off = (int64_t)M * coutp;
-    L.flags = (flags & 1 ? CONV_RELU : 0) | (flags & 4 ? CONV_RESID : 0) | (flags & (CONV_POOL | CONV_NOSTORE | CONV_RESX | CONV_FINAL));
+    L.flags = (flags & 1 ? CONV_RELU : 0) | (flags & 4 ? CONV_RESID : 0) | (flags & (CONV_POOL | CONV_NOSTORE | CONV_RESX | CONV_FINAL | CONV_RESACC));
     L.act_mode = precision == DTRAJ_PREC_TF32 ? ACT_ROUND : precision == DTRAJ_PREC_TF32X3 ? ACT_SPLIT : ACT_PLAIN;
     L.f16 = precision == DTRAJ_PREC_F16 ? 1 : 0;      // (buffers stay sized for fp32: zeros either way)
     float* aux = nullptr;      // pooled output | raw input | 1x1 weights | final weights | eps, all zero
@@ -1157,7 +1175,8 @@ extern "C" int dtraj_bench_conv(int32_t precision, int32_t c0, int32_t c1, int32
     UmmaLaunch U;
     if (precision != DTRAJ_PREC_FP32) {
         umma_set_smem_attr();
-        rc = build_umma_launch(&U, L, precision == DTRAJ_PREC_TF32X3 ? 3 : 1, dev + wo, pc.rows);
+        rc = build_umma_launch(&U, L, precision == DTRAJ_PREC_TF32X3 ? 3 : 1, dev + wo, pc.rows, resacc ? dev + wro : nullptr,
+                               resacc ? pr.rows : 0, debug == 2 ? kUmmaGeneric : debug);
     }
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
@@ -1182,22 +1201,31 @@ extern "C" int dtraj_test_conv(int32_t precision, const float* x0, int32_t c0, c
                                const float* resid, float* out, void* stream) {
     if (H != W) return fail(DTRAJ_EINVAL, "test_conv: H must equal W");
     if (ksize != 1 && ksize != 3) return fail(DTRAJ_EINVAL, "test_conv: ksize must be 1 or 3");
+    const bool resacc = (flags & 4) != 0;            // x1 feeds a fused 1x1 residual conv (CONV_RESACC), see include/dtraj.h
+    if (resacc && (precision == DTRAJ_PREC_FP32 || precision == DTRAJ_PREC_TF32X3 || !x1 || c1 < 1))
+        return fail(DTRAJ_EINVAL, "test_conv: a fused residual conv needs precision f16 or tf32 and a second input");
     cudaStream_t st = (cudaStream_t)stream;
     Arena A;
-    PackedConv pc;
-    size_t wo, bo;
-    std::vector<double> shift(cout);
+    PackedConv pc, pr;
+    size_t wo, bo, wro = 0, bro = 0;
+    std::vector<double> shift(cout), rshift(cout);
     for (int i = 0; i < cout; ++i) shift[i] = bias_host[i];
-    pack_conv(&A, &wo, &bo, &pc, w_host, cout, c0, c1, ksize, ksize == 3 && H == 1, nullptr, shift.data(), precision);
+    pack_conv(&A, &wo, &bo, &pc, w_host, cout, c0, resacc ? 0 : c1, ksize, ksize == 3 && H == 1, nullptr, shift.data(), precision);
+    if (resacc) {
+        for (int i = 0; i < cout; ++i) rshift[i] = bias_host[cout + i];
+        pack_conv(&A, &wro, &bro, &pr, w_host + (size_t)cout * c0 * ksize * ksize, cout, c1, 0, 1, false, nullptr, rshift.data(), precision);
+    }
     float* dev = nullptr;
     DTRAJ_CUDA(cudaMalloc(&dev, A.h.size() * sizeof(float)));
     DTRAJ_CUDA(cudaMemcpy(dev, A.h.data(), A.h.size() * sizeof(float), cudaMemcpyHostToDevice));
     ConvLayer L;
     memset(&L, 0, sizeof(L));
     const int64_t M = n * H * W;
-    L.src0 = x0; L.c0p = pc.c0p; L.src1 = x1; L.c1p = pc.c1p;
+    L.src0 = x0; L.c0p = pc.c0p;
+    if (resacc) { L.rsrc0 = x1; L.rc0p = pr.c0p; L.rbias = dev + bro; }
+    else { L.src1 = x1; L.c1p = pc.c1p; }
     L.H = H; L.W = W; L.M = M; L.ntaps = pc.ntaps; L.wpk = dev + wo; L.bias = dev + bo; L.coutp = pc.coutp;
-    L.resid = resid; L.out = out; L.flags = (flags & 1 ? CONV_RELU : 0) | (resid ? CONV_RESID : 0);
+    L.resid = resid; L.out = out; L.flags = (flags & 1 ? CONV_RELU : 0) | (resid ? CONV_RESID : 0) | (resacc ? CONV_RESACC : 0);
     L.act_mode = (flags & 2) ? ACT_ROUND : ACT_PLAIN;
     L.f16 = precision == DTRAJ_PREC_F16 ? 1 : 0;
     int rc = 0;
@@ -1217,7 +1245,8 @@ extern "C" int dtraj_test_conv(int32_t precision, const float* x0, int32_t c0, c
         }
         umma_set_smem_attr();
         UmmaLaunch U;
-        rc = build_umma_launch(&U, L, precision == DTRAJ_PREC_TF32X3 ? 3 : 1, dev + wo, pc.rows);
+        rc = build_umma_launch(&U, L, precision == DTRAJ_PREC_TF32X3 ? 3 : 1, dev + wo, pc.rows, resacc ? dev + wro : nullptr,
+                               resacc ? pr.rows : 0);
         if (!rc) rc = launch_conv_umma(U, st);
     }
     cudaError_t ce = cudaStreamSynchronize(st);

@@ -43,7 +43,7 @@ struct Enc1hParams {
     int C, H, W, coutp;
     int n_chunks;                // coutp / 64: K chunks of conv2
     int n_tiles, tiles_x, tiles_per_img;
-    int lg_tx, lg_tpi;           // log2(tiles_x), log2(tiles_per_img): both are powers of two (H = 16 or 32)
+    int lg_tx, lg_tpi;           // log2(tiles_x), log2(tiles_per_img): both are powers of two (H = 16, 32 or 64)
     int n_hbuf;                  // halo chunk buffers in the ring (>= 1; 2 x n_chunks when they fit)
     int acc_cols;                // TMEM columns per accumulator; layout [acc0 | acc1 | n_d1 x (D1 rows 0-127 | D1 rows 128-255)]
     int n_d1;                    // D1 buffers: 2 when 6 x acc_cols <= 512 (conv1 of tile i+2 runs while tile i is converted), else 1
@@ -680,15 +680,17 @@ struct Enc1hLaunch {
 // `w2` = conv2 weights packed by pack_conv in DTRAJ_PREC_F16 ([tap][chunk][coutp][64] halfs), `w2_rows` its 128-byte rows
 inline int build_enc1h_launch(Enc1hLaunch* E, int C, int H, int coutp, int cout_real, int64_t R, const float* w2, int64_t w2_rows) {
     memset(E, 0, sizeof(*E));
-    if (C < 1 || C > 4 || H % 16 || H > 32 || coutp % 64 || coutp > 128) return fail(DTRAJ_EINVAL, "enc1(f16): unsupported geometry");
+    if (C < 1 || C > 4 || (H != 16 && H != 32 && H != 64) || coutp % 64 || coutp > 128) return fail(DTRAJ_EINVAL, "enc1(f16): unsupported geometry");
     Enc1hParams& p = E->p;
     p.C = C; p.H = H; p.W = H; p.coutp = coutp;
     p.n_chunks = coutp / 64;
     p.n_slices = (9 * C + 2 + 15) / 16;          // 9C taps + two bias slots
     p.tiles_x = H / 8;
     p.tiles_per_img = (H / 16) * p.tiles_x;
-    p.lg_tx = H == 16 ? 1 : 2;
-    p.lg_tpi = H == 16 ? 1 : 3;
+    p.lg_tx = 0;
+    while ((1 << p.lg_tx) < p.tiles_x) ++p.lg_tx;
+    p.lg_tpi = 0;
+    while ((1 << p.lg_tpi) < p.tiles_per_img) ++p.lg_tpi;
     const int64_t nt = R * p.tiles_per_img;
     if (nt >= ((int64_t)1 << 30)) return fail(DTRAJ_EINVAL, "enc1(f16): batch too large");
     p.n_tiles = (int)nt;

@@ -363,7 +363,7 @@ struct Enc1Launch {
 // `w2` = conv2 weights packed by pack_conv ([tap][chunk][coutp][32], tf32-rounded), `w2_rows` its rows
 inline int build_enc1_launch(Enc1Launch* E, int C, int H, int coutp, int cout_real, int64_t R, const float* w2, int64_t w2_rows) {
     memset(E, 0, sizeof(*E));
-    if (C < 1 || C > 4 || H % 16 || H > 32 || coutp % 32 || coutp > 256) return fail(DTRAJ_EINVAL, "enc1: unsupported geometry");
+    if (C < 1 || C > 4 || (H != 16 && H != 32 && H != 64) || coutp % 32 || coutp > 256) return fail(DTRAJ_EINVAL, "enc1: unsupported geometry");
     Enc1Params& p = E->p;
     p.C = C; p.H = H; p.W = H; p.coutp = coutp;
     p.n_chunks = coutp / 32;

@@ -333,13 +333,15 @@ inline int launch_wasserstein(const float* T, const float* S, int64_t N, int L, 
 // words, mask to the smallest 2^k - 1 >= max, reject values > max.  The kernel below reproduces that stream bit for bit
 // (integer work: tests/test_gpu_metrics.py compares it with numpy itself): one thread per seed walks its L consecutive
 // permutations; MT state and permutation live in shared memory, interleaved over the block's threads (bank = thread).
-constexpr int kChoiceThreads = 16;
-
+// kChoiceThreads seeds per block: 16 up to D = 4096; wider frames take 8 (D <= 12288: 216 KB) or 4 (D <= 16384: 138 KB) so that
+// the interleaved uint16 permutations still fit the 227 KB of shared memory.
+template <int kChoiceThreads>
 __global__ void __launch_bounds__(kChoiceThreads) k_numpy_choice(const uint32_t* __restrict__ seeds, int n_seeds, int L, int D, int K,
                                                                  int32_t* __restrict__ out) {
+    constexpr unsigned kMask = (1u << kChoiceThreads) - 1u;
     extern __shared__ __align__(16) uint8_t ch_smem[];
-    uint32_t* mt = reinterpret_cast<uint32_t*>(ch_smem);                                   // [624][16]
-    uint16_t* perm = reinterpret_cast<uint16_t*>(ch_smem + 624 * kChoiceThreads * 4);      // [D][16]
+    uint32_t* mt = reinterpret_cast<uint32_t*>(ch_smem);                                   // [624][kChoiceThreads]
+    uint16_t* perm = reinterpret_cast<uint16_t*>(ch_smem + 624 * kChoiceThreads * 4);      // [D][kChoiceThreads]
     const int t = threadIdx.x;
     const int sidx = blockIdx.x * kChoiceThreads + t;
     const bool live = sidx < n_seeds;
@@ -384,7 +386,7 @@ __global__ void __launch_bounds__(kChoiceThreads) k_numpy_choice(const uint32_t*
                 pm[j * kChoiceThreads] = a;
             }
         }
-        __syncwarp(0xffffu);
+        __syncwarp(kMask);
         // coalesced write-out: the block's threads share the rows of each seed
         for (int s = 0; s < kChoiceThreads; ++s) {
             const int so = blockIdx.x * kChoiceThreads + s;
@@ -392,22 +394,29 @@ __global__ void __launch_bounds__(kChoiceThreads) k_numpy_choice(const uint32_t*
             int32_t* dst = out + ((size_t)so * L + f) * K;
             for (int k = t; k < K; k += kChoiceThreads) dst[k] = (int32_t)perm[k * kChoiceThreads + s];
         }
-        __syncwarp(0xffffu);
+        __syncwarp(kMask);
     }
 }
 
-inline int launch_numpy_choice(const uint32_t* seeds, int n_seeds, int L, int D, int K, int32_t* out, cudaStream_t st) {
-    if (n_seeds < 0 || L < 1 || D < 2 || D > 4096 || K < 1 || K > D) return fail(DTRAJ_EINVAL, "numpy_choice: bad argument (2 <= D <= 4096, 1 <= K <= D)");
-    if (n_seeds == 0) return 0;
-    const size_t smem = (size_t)624 * kChoiceThreads * 4 + (size_t)D * kChoiceThreads * 2;
+template <int kT>
+inline int launch_numpy_choice_t(const uint32_t* seeds, int n_seeds, int L, int D, int K, int32_t* out, int d_max, cudaStream_t st) {
+    const size_t smem = (size_t)624 * kT * 4 + (size_t)D * kT * 2;
     static bool attr_set = false;
     if (!attr_set) {
-        DTRAJ_CUDA(cudaFuncSetAttribute(k_numpy_choice, cudaFuncAttributeMaxDynamicSharedMemorySize, 624 * kChoiceThreads * 4 + 4096 * kChoiceThreads * 2));
+        DTRAJ_CUDA(cudaFuncSetAttribute(k_numpy_choice<kT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 624 * kT * 4 + d_max * kT * 2));
         attr_set = true;
     }
-    k_numpy_choice<<<(unsigned)((n_seeds + kChoiceThreads - 1) / kChoiceThreads), kChoiceThreads, smem, st>>>(seeds, n_seeds, L, D, K, out);
+    k_numpy_choice<kT><<<(unsigned)((n_seeds + kT - 1) / kT), kT, smem, st>>>(seeds, n_seeds, L, D, K, out);
     DTRAJ_LAUNCH_CHECK();
     return 0;
+}
+
+inline int launch_numpy_choice(const uint32_t* seeds, int n_seeds, int L, int D, int K, int32_t* out, cudaStream_t st) {
+    if (n_seeds < 0 || L < 1 || D < 2 || D > 16384 || K < 1 || K > D) return fail(DTRAJ_EINVAL, "numpy_choice: bad argument (2 <= D <= 16384, 1 <= K <= D)");
+    if (n_seeds == 0) return 0;
+    if (D <= 4096) return launch_numpy_choice_t<16>(seeds, n_seeds, L, D, K, out, 4096, st);
+    if (D <= 12288) return launch_numpy_choice_t<8>(seeds, n_seeds, L, D, K, out, 12288, st);
+    return launch_numpy_choice_t<4>(seeds, n_seeds, L, D, K, out, 16384, st);
 }
 
 }  // namespace dtraj

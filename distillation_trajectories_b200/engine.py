@@ -137,10 +137,15 @@ class UNetEngine:
         for ent in model.__dict__.pop("_dtraj_engines", {}).values():
             ent[1].close()
 
-    def close(self):
+    def drop_samplers(self):
+        """Destroy the cached sampling loops (captured graphs) and release their workspaces and trajectory buffers.  The caller
+        makes sure the device has finished with them."""
         for s in self._samplers.values():
             s.close()
         self._samplers = {}
+
+    def close(self):
+        self.drop_samplers()
         _live_engines.discard(self)
         if getattr(self, "handle", None):
             self.lib.dtraj_unet_destroy(self.handle)

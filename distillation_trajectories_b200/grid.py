@@ -228,6 +228,38 @@ def finish_chunk(red, w1, ck, config, sums):
     return red_h.nbytes + w1_h.nbytes
 
 
+def seeds_per_chunk_64(teacher_model, student_models, config, n_scales, precision, device, mem_fraction=0.6):
+    """64x64 sweeps only: the most seeds per chunk whose buffers fit in ``mem_fraction`` of the device's memory.  Per (seed, guidance)
+    pair and model: the forward workspace of up to two rows (CFG; dtraj_unet_workspace_bytes: about 5 MB per row of the 3x64x64
+    teacher in fp16, twice that in the TF32 modes) and the trajectory buffer of the model's captured loop; per student also the
+    contiguous copies of both trajectories that ``pair_reductions`` reduces when a frame is wider than MAX_GROUP_ELEMS.  (Measured
+    on a B200 with the teacher and the sf 0.5 student: 101.8 GB peak against about 106 GB estimated for a 512-seed fp16 chunk,
+    profiles/r03a_image64_bench.json.)  At 16x16 and 32x32 the chunk is ``max_pairs`` alone."""
+    prec = precision or te.get_precision("S2")
+    H, T = int(config.image_size), int(config.timesteps)
+    D = int(config.channels) * H * H
+    frames = (T + 2) * D * 4                          # one trajectory (x_T, T - 1 updates, the repeated last frame) + slack
+    models = {id(m): m for m in [teacher_model] + list(student_models)}
+    per_pair = 0.0
+    for m in models.values():
+        eng = te.UNetEngine.for_model(m.eval(), H, T, prec, device, verify=False)
+        per_pair += eng.workspace_bytes(2 * 1024) / 1024 + frames
+    n_students = sum(1 for m in student_models if m is not teacher_model)
+    if D > tm.MAX_GROUP_ELEMS:
+        per_pair += n_students * 2 * frames
+    budget = mem_fraction * torch.cuda.get_device_properties(device).total_memory
+    return max(1, int(budget // (per_pair * n_scales)))
+
+
+def _drop_samplers(models, device):
+    """Release the captured loops (workspaces, trajectory buffers) cached on the engines of ``models`` once the device has
+    finished with them."""
+    torch.cuda.synchronize(device)
+    for m in models:
+        for ent in m.__dict__.get("_dtraj_engines", {}).values():
+            ent[1].drop_samplers()
+
+
 @torch.no_grad()
 def sweep(teacher_model, students, config, guidance_scales, num_samples, device=None, rank=0, world_size=1,
           max_pairs=4096, precision=None, reduce=True, stats=None):
@@ -251,6 +283,9 @@ def sweep(teacher_model, students, config, guidance_scales, num_samples, device=
     sums = np.zeros((len(names), G, len(tm.SCALAR_KEYS) + 1), np.float64)
     mine = shard_samples(num_samples, rank, world_size)
     per_chunk = max(1, max_pairs // G)
+    big = int(config.image_size) == 64 and device.type == "cuda"
+    if big:
+        per_chunk = min(per_chunk, seeds_per_chunk_64(teacher_model, models, config, G, precision, device))
     pieces = [mine[c0:c0 + per_chunk] for c0 in range(0, len(mine), per_chunk)]
     n_traj = n_pairs = h2d = d2h = 0
     pending = None                                  # (readback, chunk) of the previous chunk
@@ -258,6 +293,8 @@ def sweep(teacher_model, students, config, guidance_scales, num_samples, device=
     tm_ = {"run": 0.0, "stage": 0.0, "wait": 0.0, "finish": 0.0}
     for i in range(len(pieces)):
         ck = nxt
+        if big and i > 0 and len(pieces[i]) != len(pieces[i - 1]):
+            _drop_samplers([teacher_model] + models, device)   # (64x64: the loops of the full chunks would stay cached beside the last one's)
         t0 = time.perf_counter()
         red, w1, nt = run_chunk(teacher_model, models, ck, device, precision, verify_weights=(i == 0))   # queued, not waited for
         engines = [ent[1] for m in [teacher_model] + models for ent in m.__dict__.get("_dtraj_engines", {}).values()

@@ -63,7 +63,7 @@ typedef struct dtraj_unet dtraj_unet;
 
 typedef struct {
     int32_t channels;      /* config.channels                       models.py:99           */
-    int32_t image_size;    /* H == W; 16 or 32 (multiple of 16)                            */
+    int32_t image_size;    /* H == W; 16, 32 or 64 (any other size is refused)              */
     int32_t dims[4];       /* DiffusionUNet.dims                    models.py:110          */
     int32_t temb_dim;      /* DiffusionUNet.time_emb_dim            models.py:101          */
     int32_t n_timesteps;   /* time tables cover t = 0 .. n_timesteps-1                     */
@@ -244,7 +244,7 @@ int dtraj_wasserstein(const float* teacher, const float* student,
  * bit for bit, L consecutive choice() calls per seed.
  *   seeds  dev uint32 [n_seeds]   (the value passed to np.random.seed)
  *   out    dev int32  [n_seeds, L, K]  -- directly usable as `idx` of dtraj_wasserstein
- * 2 <= D <= 4096, 1 <= K <= D.
+ * 2 <= D <= 16384, 1 <= K <= D.
  */
 int dtraj_numpy_choice_sets(const uint32_t* seeds, int32_t n_seeds, int32_t L, int32_t D, int32_t K,
                             int32_t* out, void* stream);
@@ -280,7 +280,10 @@ int dtraj_error_flag_async(uint32_t* host_flag, void* stream);
  * tests (tests/test_gpu_conv.py).  x0/x1 NHWC dev [n, H, W, c0p]/[.., c1p] (x1 may be
  * NULL); w host [Cout, c0+c1, k, k] (k = 1 or 3), bias host [Cout]; out dev NHWC
  * [n, H, W, coutp] with coutp = round_up(Cout, 32).  flags: bit0 relu, bit1 round
- * outputs to tf32.  In DTRAJ_PREC_F16 x0/x1/resid/out are __half maps with channels
+ * outputs to tf32, bit2 (DTRAJ_PREC_F16 / DTRAJ_PREC_TF32 only) x1 is not a second source of the main conv but the input of
+ * a fused 1x1 residual conv (CONV_RESACC, the decoder / enc2 conv2 form): w then holds [Cout, c0, k, k] followed by the
+ * residual weights [Cout, c1], bias holds [Cout] followed by the residual bias [Cout], and out = act(conv(x0) + bias) +
+ * conv1x1(x1) + residual bias (+ resid).  In DTRAJ_PREC_F16 x0/x1/resid/out are __half maps with channels
  * padded to 64. */
 int dtraj_test_conv(int32_t precision, const float* x0, int32_t c0, const float* x1, int32_t c1,
                     int64_t n, int32_t H, int32_t W, const float* w_host, const float* bias_host,
@@ -290,7 +293,11 @@ int dtraj_test_conv(int32_t precision, const float* x0, int32_t c0, const float*
 /* ------------------------------------------------------------------ diagnostics (tools/, not used by the package's hot path)
  * Kernel-only timing of one conv layer shape on zero-filled buffers allocated inside (tools/conv_bench.py): `iters`
  * launches between one event pair, average milliseconds in *ms_out.  flags: bit0 relu, bit2 residual input, plus the
- * CONV_POOL / CONV_NOSTORE / CONV_RESX / CONV_FINAL tail bits of csrc/conv_simt.cuh.  `debug` must be 0. */
+ * CONV_POOL / CONV_NOSTORE / CONV_RESX / CONV_FINAL / CONV_RESACC tail bits of csrc/conv_simt.cuh (CONV_RESACC: x1, c1
+ * channels, feeds the fused 1x1 residual conv instead of the main conv).  `debug` (A/B experiments): 0 = the tile form and
+ * shared-memory split the forward plan uses, 2 = the generic [image][y][x] tiles where that form is a halo form,
+ * 0x100 | n_hb << 4 | epi_bufs = the halo form with n_hb halo slots and epi_bufs epilogue buffers per warp; other values
+ * are refused. */
 int dtraj_bench_conv(int32_t precision, int32_t c0, int32_t c1, int32_t cout, int64_t n, int32_t H, int32_t ksize,
                      int32_t flags, int32_t iters, int32_t debug, float* ms_out);
 /* Peek at the library-wide error word without clearing it (tests assert it stays 0). */

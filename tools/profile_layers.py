@@ -1,6 +1,6 @@
 """GPU: per-launch device time of ONE forward + step of a captured S2 loop, for any image size / student width.
 
-    python tools/profile_layers.py <H: 16|32> <seeds> <size factors, comma separated> [precision] [w]
+    python tools/profile_layers.py <H: 16|32|64> <seeds> <size factors, comma separated> [precision] [w]
 
 Every (seed, w) pair of a model is one sample (CFG: two forward rows).  Uses dtraj_sampler_profile_text: the loop runs
 un-captured with a CUDA event pair around every launch, the table is the SECOND step's launches (warm caches, real data).
@@ -20,7 +20,13 @@ seeds = int(sys.argv[2]) if len(sys.argv) > 2 else 296
 sfs = [float(a) for a in sys.argv[3].split(",")] if len(sys.argv) > 3 else [1.0, 0.5]
 prec = sys.argv[4] if len(sys.argv) > 4 else "f16"
 scales = [float(sys.argv[5])] if len(sys.argv) > 5 else (bench.GUIDANCE if H == 16 else [7.5])
-cfg = bench.Cfg if H == 16 else bench.Cfg32
+
+
+class Cfg64(bench.Cfg):          # 3x64x64, 50 steps (the bench configs stop at 32x32)
+    channels, image_size = 3, 64
+
+
+cfg = {16: bench.Cfg, 32: bench.Cfg32, 64: Cfg64}[H]
 dev = torch.device("cuda", 0)
 ck = grid.stage_chunk(list(range(seeds)), cfg, scales, dev)
 print(f"# {cfg.channels}x{H}x{H}, {seeds} seeds x {len(scales)} scales, precision {prec}; second step of the loop, CUDA events per launch")
