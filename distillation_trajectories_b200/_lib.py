@@ -16,6 +16,7 @@ PREC_FP32, PREC_TF32, PREC_TF32X3, PREC_F16 = 0, 1, 2, 3
 VAR_NONE, VAR_COND0, VAR_COND1 = 0, 1, 2
 RULE_S1, RULE_S2, RULE_S3 = 1, 2, 3
 METRIC_Q = 6
+METRIC_Q_RAGGED = 8
 
 PRECISIONS = {"fp32": PREC_FP32, "tf32": PREC_TF32, "tf32x3": PREC_TF32X3, "f16": PREC_F16}
 
@@ -61,7 +62,9 @@ SIGNATURES = {
     "dtraj_sampler_profile": (C.c_int, [_P, _P, C.POINTER(C.c_double), C.POINTER(_I64), C.POINTER(C.c_double)]),
     "dtraj_metrics_pairs": (C.c_int, [_P, _P, _I64, _I32, _I32, _P, _P]),
     "dtraj_wasserstein": (C.c_int, [_P, _P, _I64, _I32, _I32, _P, _P, _I32, _P, _P]),
-    "dtraj_unet_forward_rows": (C.c_int, [_P, _P, _I64, _P, _P, _P, _I64, _P]),
+    "dtraj_metrics_pairs_ragged": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _P, _P, _P, _P]),
+    "dtraj_wasserstein_ragged": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _P, _P, _I32, _P, _P]),
+    "dtraj_unet_forward_rows":(C.c_int, [_P, _P, _I64, _P, _P, _P, _I64, _P]),
     "dtraj_numpy_choice_sets": (C.c_int, [_P, _I32, _I32, _I32, _I32, _P, _P]),
     "dtraj_project": (C.c_int, [_P, _I64, _I32, _P, _P, _I32, _P, _P]),
     "dtraj_sampler_flops": (C.c_int, [_P, C.POINTER(C.c_double)]),

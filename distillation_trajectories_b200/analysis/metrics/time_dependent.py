@@ -25,14 +25,22 @@ def _velocities(trajs_a, trajs_b, dev):
             _images(trajs_a[0])[0].shape == _images(trajs_b[0])[0].shape:
         red = _reduce(_stack(trajs_a, dev), _stack(trajs_b, dev))
         return _to_lists(red[:, :, 1]), _to_lists(red[:, :, 2])
-    out = []
-    for trajs in (trajs_a, trajs_b):
-        res = []
-        for t in trajs:                      # ragged: one launch per trajectory, paired with itself
-            x = _stack([t], dev)
-            res.extend(_to_lists(_reduce(x, x)[:, :, 1]))
-        out.append(res)
-    return out[0], out[1]
+    return _velocities_by_length(trajs_a, dev), _velocities_by_length(trajs_b, dev)
+
+
+def _velocities_by_length(trajs, dev):
+    """distances of one list of trajectories of different lengths: one launch per distinct (length, frame shape), each
+    trajectory paired with itself; the lists come back in input order."""
+    groups = {}
+    for k, t in enumerate(trajs):
+        im = _images(t)
+        groups.setdefault((len(im), tuple(im[0].shape)), []).append(k)
+    rows = [None] * len(trajs)
+    for ks in groups.values():
+        x = _stack([trajs[k] for k in ks], dev)
+        for k, r in zip(ks, _reduce(x, x)[:, :, 1]):
+            rows[k] = r
+    return [d for r in rows for d in _to_lists(r[None])]
 
 
 def _reduce(a, b):

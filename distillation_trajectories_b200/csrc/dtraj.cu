@@ -998,7 +998,21 @@ extern "C" int dtraj_wasserstein(const float* teacher, const float* student, int
                                  const int32_t* idx_set, int32_t K, float* out, void* stream) {
     if (N == 0) return 0;
     if (!teacher || !student || !out || N < 0 || L < 1) return fail(DTRAJ_EINVAL, "wasserstein: bad argument");
-    return launch_wasserstein(teacher, student, N, L, D, idx, idx_set, K, out, (cudaStream_t)stream);
+    return launch_wasserstein(teacher, student, N, L, L, D, idx, idx_set, K, out, (cudaStream_t)stream);
+}
+
+extern "C" int dtraj_metrics_pairs_ragged(const float* teacher, const float* student, int64_t N, int32_t LT, int32_t LS, int32_t D,
+                                          const int32_t* rs_pos, const float* rs_frac, float* out, void* stream) {
+    if (N == 0) return 0;
+    if (!teacher || !student || !rs_pos || !rs_frac || !out || N < 0) return fail(DTRAJ_EINVAL, "metrics_ragged: bad argument");
+    return launch_metrics_pairs_ragged(teacher, student, N, LT, LS, D, rs_pos, rs_frac, out, (cudaStream_t)stream);
+}
+
+extern "C" int dtraj_wasserstein_ragged(const float* teacher, const float* student, int64_t N, int32_t LT, int32_t LS, int32_t D,
+                                        const int32_t* idx, const int32_t* idx_set, int32_t K, float* out, void* stream) {
+    if (N == 0) return 0;
+    if (!teacher || !student || !out || N < 0) return fail(DTRAJ_EINVAL, "wasserstein_ragged: bad argument");
+    return launch_wasserstein(teacher, student, N, LT, LS, D, idx, idx_set, K, out, (cudaStream_t)stream);
 }
 
 extern "C" int dtraj_numpy_choice_sets(const uint32_t* seeds, int32_t n_seeds, int32_t L, int32_t D, int32_t K, int32_t* out, void* stream) {

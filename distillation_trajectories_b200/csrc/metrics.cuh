@@ -128,20 +128,183 @@ inline int launch_metrics_pairs(const float* T, const float* S, int64_t N, int L
     return 0;
 }
 
+// Teacher and student of different lengths (analysis/metrics/trajectory_metrics.py:239-279: a student sampled with
+// fewer steps than its teacher).  n = min(LT, LS); "long" is the teacher when LT >= LS, "short" the other one.
+// Same walk as k_metrics_pairs over max(LT, LS) frames: frame i of each trajectory is loaded once while i < its length and
+// the previous frame stays in registers.  The path-alignment term lerp(long[p_j], long[p_j + 1], f_j) is formed when the
+// walk holds long frames p_j and p_j + 1; short frame j is read a second time for it.  Three single frames are read once
+// more: T_0 and S_0 at each trajectory's last frame (holding them in registers for the whole walk would cost a second block
+// per SM at D = 3072), and the short trajectory's last frame for the endpoint term.  Bytes requested per pair:
+// 4 * D * (L_long + 2 * L_short + 3), against the algorithmic 4 * D * (LT + LS).
+//   out[n][i][0] = sum (T_i - S_i)^2                               (i < n)
+//   out[n][i][1] = sum (T_{i+1} - T_i)^2 (i < LT-1),  [2] = sum (S_{i+1} - S_i)^2 (i < LS-1)
+//   out[n][i][3] = sum dT_i * dS_i                                 (i < n-1)
+//   out[n][0][4] = sum (T_{LT-1} - T_0)^2,  [0][5] = sum (S_{LS-1} - S_0)^2,  [0][6] = sum (T_{LT-1} - S_{LS-1})^2
+//   out[n][j][7] = sum ((1 - f_j) long_{p_j} + f_j long_{p_j+1} - short_j)^2   (j < n)
+// every other entry of [N, max(LT, LS), 8] is 0.  Short frame j is taken once the walk has passed long frame p_j + 1
+// (p non-decreasing, 0 <= p_j <= L_long - 2), and at the last long frame at the latest.
+constexpr int kRaggedQ = 8;
+
+template <int K>
+__global__ void __launch_bounds__(256) k_metrics_pairs_ragged(const float* __restrict__ teacher, const float* __restrict__ student,
+                                                              int64_t N, int LT, int LS, int D4, int G,
+                                                              const int32_t* __restrict__ rs_pos, const float* __restrict__ rs_frac,
+                                                              float* __restrict__ out) {
+    extern __shared__ float part[];          // [pairs_per_block][Lmax][warps_per_group][5]
+    const int ppb = 256 / G, wpg = G / 32 > 0 ? G / 32 : 1;
+    const int g = threadIdx.x / G, tg = threadIdx.x % G;
+    const int warp_in_group = tg >> 5, lane = threadIdx.x & 31;
+    const int64_t n = (int64_t)blockIdx.x * ppb + g;
+    const bool active = n < N;
+    const int Lmax = LT > LS ? LT : LS, Ln = LT < LS ? LT : LS;
+    const bool t_long = LT >= LS;
+    float* mypart = part + (size_t)g * Lmax * wpg * 5;
+    float4 prevT[K], prevS[K], nxtT[K], nxtS[K], sh[K];
+    const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4* Tb = reinterpret_cast<const float4*>(teacher) + (active ? n : 0) * (int64_t)LT * D4;
+    const float4* Sb = reinterpret_cast<const float4*>(student) + (active ? n : 0) * (int64_t)LS * D4;
+    const float4* Shb = t_long ? Sb : Tb;
+    auto load = [&](const float4* base, int i, bool ok, float4* v) {
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const int e = tg + k * G;
+            v[k] = (ok && active && e < D4) ? ld_stream4(reinterpret_cast<const float*>(base + (int64_t)i * D4 + e)) : zero4;
+        }
+    };
+    auto sq4 = [](float4 a) { return a.x * a.x + a.y * a.y + a.z * a.z + a.w * a.w; };
+    auto sub4 = [](float4 a, float4 b) { return make_float4(a.x - b.x, a.y - b.y, a.z - b.z, a.w - b.w); };
+    auto dot4 = [](float4 a, float4 b) { return a.x * b.x + a.y * b.y + a.z * b.z + a.w * b.w; };
+    auto lerp4 = [](float4 a, float4 b, float f) {   // exact at f = 0 and f = 1
+        const float e = 1.f - f;
+        return make_float4(e * a.x + f * b.x, e * a.y + f * b.y, e * a.z + f * b.z, e * a.w + f * b.w);
+    };
+
+    load(Tb, 0, true, nxtT);
+    load(Sb, 0, true, nxtS);
+    float endT = 0.f, endS = 0.f, endTS = 0.f;
+    int j = 0;                               // next short frame of the path-alignment term
+    for (int i = 0; i < Lmax; ++i) {
+        float4 curT[K], curS[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) { curT[k] = nxtT[k]; curS[k] = nxtS[k]; }
+        load(Tb, i + 1, i + 1 < LT, nxtT);
+        load(Sb, i + 1, i + 1 < LS, nxtS);
+        const bool inT = i < LT, inS = i < LS;
+        float d2 = 0.f, vt2 = 0.f, vs2 = 0.f, dot = 0.f;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            d2 += sq4(sub4(curT[k], curS[k]));
+            if (i > 0) {
+                const float4 dt = sub4(curT[k], prevT[k]), ds = sub4(curS[k], prevS[k]);
+                vt2 += sq4(dt); vs2 += sq4(ds); dot += dot4(dt, ds);
+            }
+        }
+        if (i == LT - 1) {                   // frame 0 is re-read rather than held in registers for the whole walk
+            load(Tb, 0, true, sh);
+#pragma unroll
+            for (int k = 0; k < K; ++k) endT += sq4(sub4(curT[k], sh[k]));
+        }
+        if (i == LS - 1) {
+            load(Sb, 0, true, sh);
+#pragma unroll
+            for (int k = 0; k < K; ++k) endS += sq4(sub4(curS[k], sh[k]));
+        }
+        if (i == Lmax - 1) {                 // the long trajectory's last frame against the short one's (re-read)
+            load(Shb, Ln - 1, true, sh);
+#pragma unroll
+            for (int k = 0; k < K; ++k) endTS += sq4(sub4(t_long ? curT[k] : curS[k], sh[k]));
+        }
+        // path alignment: every short frame j whose interval [p_j, p_j + 1] ends at this long frame
+        while (i > 0 && j < Ln && (__ldg(rs_pos + j) <= i - 1 || i == Lmax - 1)) {
+            const float f = __ldg(rs_frac + j);
+            load(Shb, j, true, sh);
+            float r2 = 0.f;
+#pragma unroll
+            for (int k = 0; k < K; ++k)
+                r2 += t_long ? sq4(sub4(lerp4(prevT[k], curT[k], f), sh[k])) : sq4(sub4(lerp4(prevS[k], curS[k], f), sh[k]));
+            r2 = warp_sum(r2);
+            if (lane == 0) mypart[(j * wpg + warp_in_group) * 5 + 4] = r2;
+            ++j;
+        }
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            if (inT) prevT[k] = curT[k];
+            if (inS) prevS[k] = curS[k];
+        }
+        d2 = warp_sum(d2); vt2 = warp_sum(vt2); vs2 = warp_sum(vs2); dot = warp_sum(dot);
+        if (lane == 0) {
+            mypart[(i * wpg + warp_in_group) * 5 + 0] = d2;
+            if (i > 0) {                     // step (i-1 -> i) belongs to frame index i-1
+                float* q = mypart + ((i - 1) * wpg + warp_in_group) * 5;
+                q[1] = vt2; q[2] = vs2; q[3] = dot;
+            }
+        }
+    }
+    endT = warp_sum(endT); endS = warp_sum(endS); endTS = warp_sum(endTS);
+    __shared__ float endpart[8][3];
+    if (lane == 0) { endpart[threadIdx.x >> 5][0] = endT; endpart[threadIdx.x >> 5][1] = endS; endpart[threadIdx.x >> 5][2] = endTS; }
+    __syncthreads();
+    if (!active) return;
+    float* o = out + n * (int64_t)Lmax * kRaggedQ;
+    for (int e = tg; e < Lmax * kRaggedQ; e += G) {
+        const int i = e / kRaggedQ, q = e % kRaggedQ;
+        float s = 0.f;
+        if (q >= 4 && q <= 6) {
+            if (i == 0) for (int w = 0; w < wpg; ++w) s += endpart[g * wpg + w][q - 4];
+        } else {
+            const int c = q == 7 ? 4 : q;
+            const bool valid = q == 0 ? i < Ln : q == 1 ? i < LT - 1 : q == 2 ? i < LS - 1 : q == 3 ? i < Ln - 1 : i < Ln;
+            if (valid) for (int w = 0; w < wpg; ++w) s += mypart[(i * wpg + w) * 5 + c];
+        }
+        o[e] = s;
+    }
+}
+
+inline int launch_metrics_pairs_ragged(const float* T, const float* S, int64_t N, int LT, int LS, int D,
+                                       const int32_t* rs_pos, const float* rs_frac, float* out, cudaStream_t st) {
+    if (D % 4 != 0 || D <= 0 || LT < 1 || LS < 1 || (LT < 2 && LS < 2))
+        return fail(DTRAJ_EINVAL, "metrics_ragged: D=%d must be a positive multiple of 4, LT=%d, LS=%d >= 1 and one of them >= 2", D, LT, LS);
+    const int D4 = D / 4;
+    int G = 32;
+    while (G < 256 && (D4 + G - 1) / G > 3) G *= 2;
+    const int K = (D4 + G - 1) / G;
+    if (K > 4) return fail(DTRAJ_EINVAL, "metrics_ragged: D=%d too large (max 4096)", D);
+    const int ppb = 256 / G, wpg = G / 32, Lmax = LT > LS ? LT : LS;
+    const size_t smem = (size_t)ppb * Lmax * wpg * 5 * sizeof(float);
+    if (smem > 200 * 1024) return fail(DTRAJ_EINVAL, "metrics_ragged: max(LT, LS)=%d too large", Lmax);
+    if (N == 0) return 0;
+    const unsigned grid = (unsigned)((N + ppb - 1) / ppb);
+#define DTRAJ_MPR(KK)                                                                             \
+    {                                                                                             \
+        if (smem > 48 * 1024)                                                                     \
+            DTRAJ_CUDA(cudaFuncSetAttribute(k_metrics_pairs_ragged<KK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        k_metrics_pairs_ragged<KK><<<grid, 256, smem, st>>>(T, S, N, LT, LS, D4, G, rs_pos, rs_frac, out); \
+    }
+    switch (K) {
+        case 1: DTRAJ_MPR(1); break;
+        case 2: DTRAJ_MPR(2); break;
+        case 3: DTRAJ_MPR(3); break;
+        default: DTRAJ_MPR(4); break;
+    }
+#undef DTRAJ_MPR
+    DTRAJ_LAUNCH_CHECK();
+    return 0;
+}
+
 // 1-d Wasserstein distance between K gathered elements of T_i and S_i: for equal-size
 // samples W1 = mean |sort(u) - sort(v)| (scipy.stats.wasserstein_distance evaluates the
 // same quantity through the two CDFs).  One CTA per (pair, frame): gather -> bitonic sort
 // of both arrays in shared memory -> f64 sum of |a - b|.
 __global__ void __launch_bounds__(256) k_wasserstein(const float* __restrict__ teacher, const float* __restrict__ student,
-                                                     int L, int D, const int32_t* __restrict__ idx,
+                                                     int L, int LT, int LS, int D, const int32_t* __restrict__ idx,
                                                      const int32_t* __restrict__ idx_set, int K, int P,
                                                      float* __restrict__ out) {
     extern __shared__ float sv[];   // [2][P]
     const int64_t pf = blockIdx.x;  // n*L + i
     const int64_t n = pf / L;
     const int i = (int)(pf % L);
-    const float* t = teacher + pf * D;
-    const float* s = student + pf * D;
+    const float* t = teacher + (n * LT + i) * D;
+    const float* s = student + (n * LS + i) * D;
     const int32_t* ix = idx ? idx + ((int64_t)(idx_set ? idx_set[n] : 0) * L + i) * K : nullptr;
     for (int k = threadIdx.x; k < P; k += blockDim.x) {
         float a = INFINITY, b = INFINITY;
@@ -214,15 +377,15 @@ __device__ __forceinline__ void warp_bitonic_sort(float (&v)[E], int lane) {
 
 template <int E>
 __global__ void __launch_bounds__(256) k_wasserstein_warp(const float* __restrict__ teacher, const float* __restrict__ student,
-                                                          int64_t NL, int L, int D, const int32_t* __restrict__ idx,
+                                                          int64_t NL, int L, int LT, int LS, int D, const int32_t* __restrict__ idx,
                                                           const int32_t* __restrict__ idx_set, int K, float* __restrict__ out) {
     const int lane = threadIdx.x & 31;
     const int64_t pf = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);    // n*L + i
     if (pf >= NL) return;
     const int64_t n = pf / L;
     const int i = (int)(pf - n * L);
-    const float* t = teacher + pf * D;
-    const float* s = student + pf * D;
+    const float* t = teacher + (n * LT + i) * D;
+    const float* s = student + (n * LS + i) * D;
     const int32_t* ix = idx ? idx + ((int64_t)(idx_set ? idx_set[n] : 0) * L + i) * K : nullptr;
     float a[E], b[E];
 #pragma unroll
@@ -298,8 +461,12 @@ inline int launch_project(const float* x, int64_t F, int D, const float* comps, 
     return 0;
 }
 
-inline int launch_wasserstein(const float* T, const float* S, int64_t N, int L, int D, const int32_t* idx,
+// Frames i < L = min(LT, LS) of pairs whose teacher holds LT frames and student LS frames ([N, LT, D] / [N, LS, D], read in
+// place); idx is [n_sets, L, K] and out [N, L].  LT == LS is the equal-length form.
+inline int launch_wasserstein(const float* T, const float* S, int64_t N, int LT, int LS, int D, const int32_t* idx,
                               const int32_t* idx_set, int K, float* out, cudaStream_t st) {
+    const int L = LT < LS ? LT : LS;
+    if (L < 1) return fail(DTRAJ_EINVAL, "wasserstein: LT=%d and LS=%d must be >= 1", LT, LS);
     if (K < 1 || K > D || K > 4096) return fail(DTRAJ_EINVAL, "wasserstein: K=%d out of range (D=%d)", K, D);
     if (!idx && K != D) return fail(DTRAJ_EINVAL, "wasserstein: idx == NULL requires K == D");
     if (N * L > 0x7fffffffLL) return fail(DTRAJ_EINVAL, "wasserstein: N*L too large for one launch");
@@ -309,16 +476,16 @@ inline int launch_wasserstein(const float* T, const float* S, int64_t N, int L, 
     const int64_t NL = N * L;
     const unsigned wgrid = (unsigned)((NL + 7) / 8);
     if (P <= 256) {
-        k_wasserstein_warp<8><<<wgrid, 256, 0, st>>>(T, S, NL, L, D, idx, idx_set, K, out);
+        k_wasserstein_warp<8><<<wgrid, 256, 0, st>>>(T, S, NL, L, LT, LS, D, idx, idx_set, K, out);
         DTRAJ_LAUNCH_CHECK();
         return 0;
     }
     if (P <= 1024) {
-        k_wasserstein_warp<32><<<wgrid, 256, 0, st>>>(T, S, NL, L, D, idx, idx_set, K, out);
+        k_wasserstein_warp<32><<<wgrid, 256, 0, st>>>(T, S, NL, L, LT, LS, D, idx, idx_set, K, out);
         DTRAJ_LAUNCH_CHECK();
         return 0;
     }
-    k_wasserstein<<<(unsigned)(N * L), 256, 2 * P * sizeof(float), st>>>(T, S, L, D, idx, idx_set, K, P, out);
+    k_wasserstein<<<(unsigned)(N * L), 256, 2 * P * sizeof(float), st>>>(T, S, L, LT, LS, D, idx, idx_set, K, P, out);
     DTRAJ_LAUNCH_CHECK();
     return 0;
 }

@@ -18,7 +18,6 @@ from .. import sampling
 from . import trajectory_store as store
 from ..engine import UNetEngine, check_device_errors, get_precision
 from ..analysis.metrics import trajectory_metrics as tm
-from ..analysis.metrics.trajectory_metrics import compute_trajectory_metrics
 
 
 class TrajectoryManager:
@@ -180,10 +179,11 @@ class TrajectoryManager:
                "mean_directional_consistency", "mean_position_difference", "distribution_similarity"]
         allm = {k: [] for k in list(lists) + new + ["architecture_type"]}
         for i in range(0, len(names), batch_size):
+            pairs = []
             for n in names[i:i + batch_size]:
                 with open(os.path.join(self.config.trajectory_dir, n), "rb") as f:
-                    t, s = pickle.load(f)
-                m = compute_trajectory_metrics(t, s, self.config)
+                    pairs.append(pickle.load(f))
+            for m in tm.compute_trajectory_metrics_many(pairs):
                 for dst, src in lists.items():
                     allm[dst].append(m[src])
                 for k in new:
@@ -200,36 +200,19 @@ class TrajectoryManager:
         return allm
 
     def _pack_metrics(self, pack, allm, lists, new, batch_size):
-        """Metrics of every pair of a pack.  Equal-length pairs go through the batched kernels (one launch per
-        ``batch_size`` x 64 pairs) with the Wasserstein subsamples drawn from the global numpy RNG in the
-        reference's order (pair by pair, frame by frame, trajectory_metrics.py:301-306); other packs fall back
-        to the per-pair entry point."""
+        """Metrics of every pair of a pack, equal or unequal teacher / student lengths, through the batched kernels
+        (one launch per ``batch_size`` x 64 pairs) with the Wasserstein subsamples drawn from the global numpy RNG in
+        the reference's order (pair by pair, frame by frame, trajectory_metrics.py:301-306)."""
         T, S = pack["teacher"], pack["student"]
-        N, L = T.shape[0], T.shape[1]
-        if S.shape[1] != L:
-            tl, sl = store.as_reference_lists(pack, lambda a: torch.from_numpy(a).to(self.device))
-            for t, s_ in zip(tl, sl):
-                m = compute_trajectory_metrics(t, s_, self.config)
-                for dst, src in lists.items():
-                    allm[dst].append(m[src])
-                for k in new:
-                    allm[k].append(m[k])
-            return
+        N, LT, LS = T.shape[0], T.shape[1], S.shape[1]
         D, pixels = int(np.prod(T.shape[2:])), T.shape[3] * T.shape[4]
-        K = min(1000, D)
         step = max(1, batch_size) * 64
         for n0 in range(0, N, step):
             n1 = min(N, n0 + step)
-            t = torch.from_numpy(np.ascontiguousarray(T[n0:n1])).to(self.device).reshape(n1 - n0, L, D)
-            s_ = torch.from_numpy(np.ascontiguousarray(S[n0:n1])).to(self.device).reshape(n1 - n0, L, D)
-            red = tm.pair_reductions(t, s_).cpu().numpy()
-            if K == D:
-                w1 = tm.wasserstein_frames(t, s_)
-            else:
-                idx = np.stack([np.stack([np.random.choice(D, K, replace=False) for _ in range(L)])
-                                for _ in range(n1 - n0)]).astype(np.int32)
-                w1 = tm.wasserstein_frames(t, s_, torch.from_numpy(idx), torch.arange(n1 - n0, dtype=torch.int32))
-            sm = tm.scalar_metrics_batched(red, w1.cpu().numpy(), pixels, D)
+            t = torch.from_numpy(np.ascontiguousarray(T[n0:n1])).to(self.device).reshape(n1 - n0, LT, D)
+            s_ = torch.from_numpy(np.ascontiguousarray(S[n0:n1])).to(self.device).reshape(n1 - n0, LS, D)
+            idx = np.stack([tm.draw_index_sets(min(LT, LS), D) for _ in range(n1 - n0)])
+            sm = tm.pair_metrics(t, s_, idx, pixels)
             for j in range(n1 - n0):
                 for dst, src in lists.items():
                     allm[dst].append([float(v) for v in sm["_wasserstein"][j]] if src == "wasserstein_distances"

@@ -237,6 +237,42 @@ int dtraj_wasserstein(const float* teacher, const float* student,
                       float* out, void* stream);
 
 /*
+ * Teacher and student trajectories of different lengths, N pairs in one launch: the branch of
+ * compute_trajectory_metrics for len(teacher) != len(student) (trajectory_metrics.py:239-279; a
+ * student sampled with fewer steps than its teacher).  n = min(LT, LS); "long" is the teacher when
+ * LT >= LS and the student otherwise, "short" the other one.
+ *   teacher  dev [N, LT, D] fp32,  student  dev [N, LS, D] fp32 (D = C*H*W, a multiple of 4, at most 4096)
+ *   rs_pos   dev int32 [n], rs_frac dev fp32 [n]: the path-alignment resampling table, the same for
+ *            every pair -- short frame j is compared with (1 - f_j) long[p_j] + f_j long[p_j + 1],
+ *            np.interp's rule on linspace(0, 1, L) axes (p non-decreasing, 0 <= p_j <= L_long - 2)
+ *   out      dev [N, max(LT, LS), 8] fp32:
+ *        [i][0] = sum (T_i - S_i)^2                     (i < n)
+ *        [i][1] = sum (T_{i+1} - T_i)^2  (i < LT-1),  [i][2] = sum (S_{i+1} - S_i)^2  (i < LS-1)
+ *        [i][3] = sum (T_{i+1}-T_i)(S_{i+1}-S_i)        (i < n-1)
+ *        [0][4] = sum (T_{LT-1} - T_0)^2,  [0][5] = sum (S_{LS-1} - S_0)^2
+ *        [0][6] = sum (T_{LT-1} - S_{LS-1})^2           endpoint distance / mse numerator
+ *        [j][7] = sum ((1 - f_j) long_{p_j} + f_j long_{p_j+1} - short_j)^2   (j < n) path alignment
+ *        every other entry is 0.
+ * The long trajectory is read once, the short one twice, and three single frames (T_0, S_0 and the
+ * short one's last) once more: 4 * N * D * (L_long + 2 * L_short + 3) bytes requested, against the
+ * algorithmic 4 * N * D * (LT + LS).
+ * LT == LS is accepted (then the alignment term equals [j][0]); max(LT, LS) >= 2.
+ */
+int dtraj_metrics_pairs_ragged(const float* teacher, const float* student,
+                               int64_t N, int32_t LT, int32_t LS, int32_t D,
+                               const int32_t* rs_pos, const float* rs_frac, float* out, void* stream);
+
+/*
+ * dtraj_wasserstein for teacher [N, LT, D] and student [N, LS, D] of different lengths: the
+ * distances of the first n = min(LT, LS) frames (trajectory_metrics.py:296-312 zips the two frame
+ * lists), read in place.  idx dev int32 [n_idx_sets, n, K]; out dev [N, n] fp32.
+ */
+int dtraj_wasserstein_ragged(const float* teacher, const float* student,
+                             int64_t N, int32_t LT, int32_t LS, int32_t D,
+                             const int32_t* idx, const int32_t* idx_set, int32_t K,
+                             float* out, void* stream);
+
+/*
  * The subsample index sets compute_trajectory_metrics draws for frames larger than 1000 elements
  * (trajectory_metrics.py:301-306: np.random.choice(D, K, replace=False) per frame, from the global numpy RNG that
  * compare_trajectories' callers left at seed + 1, analysis/trajectory_engine.py:91-93), generated on the device: numpy's
