@@ -77,6 +77,8 @@ SIGNATURES = {
     "dtraj_debug_umma_error": (C.c_uint, []),
     "dtraj_test_conv": (C.c_int, [_I32, _P, _I32, _P, _I32, _I64, _I32, _I32, _P, _P, _I32, _I32, _I32,
                                   _P, _P, _P]),
+    "dtraj_test_plan_describe": (C.c_int, [_P, _I64, _P, _I64, _I32, C.c_char_p, _I64]),
+    "dtraj_test_plan_run": (C.c_int, [_P, _P, _I64, _I32, _P, _I32, _P, _I64, _I32, _I32, _I32, _P]),
 }
 
 _lib = None

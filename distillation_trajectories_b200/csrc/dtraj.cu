@@ -398,10 +398,14 @@ struct Launch {
     } rs;
 };
 
+// plan_build options (dtraj_test_plan_*; the product always builds with 0)
+constexpr int kPlanNoEnc1 = 1;      // k_conv_first + the generic enc1.conv2 (RESX tails) instead of the fused enc1 kernel
+
 struct dtraj_plan {
     const dtraj_unet* u = nullptr;
     int64_t R = 0;
     float* ws = nullptr;
+    int options = 0;
     // buffers (float offsets into ws); lo planes follow at +size when act_mode == ACT_SPLIT
     struct Buf { float* p = nullptr; int64_t n = 0; int64_t lo = 0; };
     Buf tmp_h, tmp_r, tmp_x, p1, x2, p2, x3, p3, x4, p4, u3, u2, u1, y1, elow;
@@ -520,13 +524,13 @@ int add_conv(dtraj_plan* P, const char* name, const PackedConv& pc, const dtraj_
     return 0;
 }
 
-int plan_build(const dtraj_unet* u, int64_t R, void* ws, int64_t ws_bytes, dtraj_plan** out) {
+int plan_build(const dtraj_unet* u, int64_t R, void* ws, int64_t ws_bytes, dtraj_plan** out, int options = 0) {
     if (R < 1) return fail(DTRAJ_EINVAL, "n_rows must be >= 1");
     const int64_t need = plan_floats(u, R, nullptr) * 4;
     if (ws_bytes < need) return fail(DTRAJ_ENOMEM, "workspace %lld B < required %lld B", (long long)ws_bytes, (long long)need);
     if (((uintptr_t)ws & 255) != 0) return fail(DTRAJ_EINVAL, "workspace must be 256-byte aligned");
     dtraj_plan* P = new dtraj_plan();
-    P->u = u; P->R = R; P->ws = (float*)ws;
+    P->u = u; P->R = R; P->ws = (float*)ws; P->options = options;
     plan_floats(u, R, P);
     const int* S = u->sizes;
     const int* dp = u->dp;
@@ -600,6 +604,7 @@ int plan_build(const dtraj_unet* u, int64_t R, void* ws, int64_t ws_bytes, dtraj
     bool fuse_enc1 = fused && S[0] % 16 == 0 && C <= 4;   // k_enc1_umma / k_enc1_f16 replace k_conv_first + the enc1.conv2 launch
     if (f16 && dp[0] > 128) fuse_enc1 = false;   // the fp16 fused kernel holds D1 + two accumulators in TMEM: widths up to 128;
                                                  // wider first blocks take k_conv_first + the generic conv2 (RESX + POOL tails)
+    if (options & kPlanNoEnc1) fuse_enc1 = false;   // (that path for the narrower first blocks every supported model has)
     auto enc1_fused = [&](Launch& l, auto& E) {   // what the two fused enc1 launches (Enc1hLaunch, Enc1Launch) share
         auto& e = E.p;
         e.w3 = u->fw3; e.b3 = u->fb3; e.rw1 = u->fw1; e.rb1 = u->fb1; e.bias2 = blk(0).conv2.bias;
@@ -715,14 +720,15 @@ int launch_record(Launch& l, const dtraj_unet* u, const float* x, int64_t x_stri
     return 0;
 }
 
-// Enqueue one U-Net forward (models.py:159-224 up to the half-resolution eps map).
+// Enqueue one U-Net forward (models.py:159-224 up to the half-resolution eps map), or its launches [first, last) (test hook).
 // `per_row`: row_variant holds t_i * 3 + variant_i (a row of the whole table) instead of the variant alone, `t` is 0.
 int plan_forward(dtraj_plan* P, const float* x, int64_t x_stride, const int32_t* row_sample, const int32_t* row_variant, int t,
-                 bool per_row, cudaStream_t st, Profiler* prof = nullptr) {
+                 bool per_row, cudaStream_t st, Profiler* prof = nullptr, size_t first = 0, size_t last = SIZE_MAX) {
     const dtraj_unet* u = P->u;
     if (t < 0 || t >= u->d.n_timesteps) return fail(DTRAJ_EINVAL, "timestep %d outside the time table (0..%d)", t, u->d.n_timesteps - 1);
     const float* trow = u->table + (size_t)t * 3 * u->tb_stride;
-    for (Launch& l : P->launches) {
+    for (size_t i = first; i < std::min(last, P->launches.size()); ++i) {
+        Launch& l = P->launches[i];
         const float* tb = l.tb_block >= 0 ? trow + u->tb_off[l.tb_block] : nullptr;
         if (prof) prof->begin(l.cls, l.name, l.grid, l.flops);
         const int rc = launch_record(l, u, x, x_stride, row_sample, row_variant, tb, per_row, st);
@@ -732,13 +738,19 @@ int plan_forward(dtraj_plan* P, const float* x, int64_t x_stride, const int32_t*
     return 0;
 }
 
+// the handle's cached plan for this batch, workspace and option set, (re)built when one of them changes
+int cached_plan(dtraj_unet* u, int64_t n_rows, void* workspace, int64_t workspace_bytes, int options) {
+    if (!u->plan || u->plan->R != n_rows || u->plan->ws != (float*)workspace || u->plan->options != options) {
+        if (u->plan) { delete u->plan; u->plan = nullptr; }
+        DTRAJ_TRY(plan_build(u, n_rows, workspace, workspace_bytes, &u->plan, options));
+    }
+    return 0;
+}
+
 // dtraj_unet_forward*: (re)build the handle's cached plan for this batch and workspace, run it, expand eps to full resolution
 int unet_forward(dtraj_unet* u, const float* x, int64_t n_rows, int t, const int32_t* row_variant, bool per_row, float* eps,
                  void* workspace, int64_t workspace_bytes, cudaStream_t st) {
-    if (!u->plan || u->plan->R != n_rows || u->plan->ws != (float*)workspace) {
-        if (u->plan) { delete u->plan; u->plan = nullptr; }
-        DTRAJ_TRY(plan_build(u, n_rows, workspace, workspace_bytes, &u->plan));
-    }
+    DTRAJ_TRY(cached_plan(u, n_rows, workspace, workspace_bytes, 0));
     const int C = u->d.channels, H = u->d.image_size;
     DTRAJ_TRY(plan_forward(u->plan, x, (int64_t)C * H * H, nullptr, row_variant, t, per_row, st));
     const int64_t n = n_rows * C * H * H;
@@ -1208,6 +1220,146 @@ extern "C" int dtraj_bench_conv(int32_t precision, int32_t c0, int32_t c1, int32
     if (ce != cudaSuccess) return fail(DTRAJ_ECUDA, "bench_conv -> %s", cudaGetErrorString(ce));
     *ms_out = ms / iters;
     return 0;
+}
+
+namespace {
+const char* const kKindNames[] = {"ENC1H", "ENC1", "FIRST", "CONV_UMMA", "CONV_SIMT", "POOL", "POOL_H", "UP", "UP_H", "UP_H4", "FINAL"};
+
+// Text form of a plan (dtraj_test_plan_describe).  Every tensor a launch reads or writes is named by the plan buffer its pointer
+// points at, so the description is derived from the records themselves; a pointer into no buffer is an error.
+struct PlanText {
+    const dtraj_plan* P;
+    std::string s;
+    int rc = 0;
+    void put(const char* fmt, ...) {
+        char line[512];
+        va_list ap;
+        va_start(ap, fmt);
+        vsnprintf(line, sizeof(line), fmt, ap);
+        va_end(ap);
+        s += line;
+    }
+    std::vector<std::pair<const char*, const dtraj_plan::Buf*>> bufs() const {
+        return {{"tmp_h", &P->tmp_h}, {"tmp_r", &P->tmp_r}, {"tmp_x", &P->tmp_x}, {"p1", &P->p1}, {"x2", &P->x2}, {"p2", &P->p2},
+                {"x3", &P->x3}, {"p3", &P->p3}, {"x4", &P->x4}, {"p4", &P->p4}, {"u3", &P->u3}, {"u2", &P->u2}, {"u1", &P->u1},
+                {"y1", &P->y1}, {"elow", &P->elow}};
+    }
+    bool half_buf(const dtraj_plan::Buf* b) const { return P->u->d.precision == DTRAJ_PREC_F16 && b != &P->elow; }
+    // one tensor of launch i: `role`, in / out, map size S, padded channels cp; p == nullptr names the raw frames x
+    void tensor(int i, const char* role, const char* dir, const void* p, int S, int cp) {
+        const char* name = "x";
+        bool half = false;
+        if (p) {
+            name = nullptr;
+            for (auto& b : bufs())
+                if (b.second->p == p) { name = b.first; half = half_buf(b.second); }
+            if (!name) { rc = fail(DTRAJ_EINVAL, "plan_describe: launch %d %s points into no plan buffer", i, role); return; }
+        }
+        put("tensor i=%d role=%s dir=%s buf=%s S=%d cp=%d type=%s\n", i, role, dir, name, S, cp, half ? "f16" : "f32");
+    }
+    void conv(int i, const ConvLayer& L) {
+        tensor(i, "src0", "in", L.src0, L.H, L.c0p);
+        if (L.src1) tensor(i, "src1", "in", L.src1, L.H, L.c1p);
+        if (L.flags & CONV_RESID) tensor(i, "resid", "in", L.resid, L.H, L.coutp);
+        if (L.flags & CONV_RESACC) {
+            tensor(i, "rsrc0", "in", L.rsrc0, L.H, L.rc0p);
+            if (L.rsrc1) tensor(i, "rsrc1", "in", L.rsrc1, L.H, L.rc1p);
+        }
+        if (L.flags & CONV_RESX) tensor(i, "x", "in", nullptr, L.H, L.xC);
+        if (!(L.flags & CONV_NOSTORE)) tensor(i, "out", "out", L.out, L.H, L.coutp);
+        if (L.flags & CONV_POOL) tensor(i, "pool", "out", L.pool_out, L.H / 2, L.coutp);
+        if (L.flags & CONV_FINAL) tensor(i, "elow", "out", L.elow, L.H, L.finC);
+    }
+    void build() {
+        const dtraj_unet* u = P->u;
+        const bool f16 = u->d.precision == DTRAJ_PREC_F16;
+        put("plan R=%lld options=%d precision=%d launches=%zu\n", (long long)P->R, P->options, u->d.precision, P->launches.size());
+        for (auto& b : bufs()) {
+            const int64_t esz = half_buf(b.second) ? 2 : 4;
+            put("buf name=%s off=%lld bytes=%lld lo=%lld type=%s\n", b.first, (long long)((b.second->p - P->ws) * 4),
+                (long long)(b.second->n * esz * (b.second->lo ? 2 : 1)), (long long)(b.second->lo * 4), esz == 2 ? "f16" : "f32");
+        }
+        for (size_t k = 0; k < P->launches.size() && !rc; ++k) {
+            const Launch& l = P->launches[k];
+            const int i = (int)k;
+            const auto& r = l.rs;
+            const char* form = "none";
+            int flags = 0, act = 0, pair = 0, split = 1, nblk = 0, epi = 0;
+            if (l.kind == Launch::CONV_UMMA) {
+                const UmmaConv& c = l.U.conv;
+                form = c.posm ? "posm" : c.halo == 1 ? "halo1" : c.halo == 2 ? "halo2" : "generic";
+                flags = c.L.flags; act = c.L.act_mode; pair = c.pair; split = c.n_split; nblk = c.nblk_img; epi = epi_kind_of(c.L.flags);
+            } else if (l.kind == Launch::CONV_SIMT) {
+                flags = l.L.flags; act = l.L.act_mode;
+            } else if (l.kind == Launch::ENC1H) {
+                pair = l.enc1h.pair;
+            } else if (l.kind == Launch::ENC1) {
+                pair = l.enc1.pair; act = l.enc1.p.act_mode;
+            } else if (l.kind == Launch::FIRST) {
+                act = l.first.act_mode;
+            } else if (l.kind != Launch::FINAL) {
+                act = r.act_mode;
+            }
+            put("launch i=%d kind=%s grid=%u flags=%d act=%d tb=%d form=%s pair=%d split=%d nblk=%d epi=%d name=%s\n", i,
+                kKindNames[l.kind], l.grid, flags, act, l.tb_block, form, pair, split, nblk, epi, l.name);
+            const int S0 = u->sizes[0], C = u->d.channels, cv = f16 ? 8 : 4;
+            switch (l.kind) {
+            case Launch::ENC1H:
+                tensor(i, "x", "in", nullptr, S0, C);
+                tensor(i, "pool", "out", l.enc1h.p.pool_out, S0 / 2, l.enc1h.p.coutp);
+                break;
+            case Launch::ENC1:
+                tensor(i, "x", "in", nullptr, S0, C);
+                tensor(i, "pool", "out", l.enc1.p.pool_out, S0 / 2, l.enc1.p.coutp);
+                break;
+            case Launch::FIRST:
+                tensor(i, "x", "in", nullptr, S0, C);
+                tensor(i, "out", "out", l.first.h, S0, l.first.coutp);
+                if (l.first.r) tensor(i, "res", "out", l.first.r, S0, l.first.coutp);
+                break;
+            case Launch::CONV_UMMA: conv(i, l.U.conv.L); break;
+            case Launch::CONV_SIMT: conv(i, l.L); break;
+            case Launch::POOL: case Launch::POOL_H:
+                tensor(i, "src0", "in", r.in, 2 * r.S, r.cv * cv);
+                tensor(i, "out", "out", r.out, r.S, r.cv * cv);
+                break;
+            case Launch::UP: case Launch::UP_H: case Launch::UP_H4:
+                tensor(i, "src0", "in", r.in, r.S, r.cv * cv);
+                tensor(i, "out", "out", r.out, 2 * r.S, r.cv * cv);
+                break;
+            case Launch::FINAL:
+                tensor(i, "src0", "in", r.in, u->sizes[1], r.cv);
+                tensor(i, "elow", "out", r.out, u->sizes[1], C);
+                break;
+            }
+        }
+    }
+};
+}  // namespace
+
+extern "C" int dtraj_test_plan_describe(dtraj_unet* u, int64_t n_rows, void* workspace, int64_t workspace_bytes, int32_t options,
+                                        char* buf, int64_t buf_len) {
+    if (!u || !workspace || !buf || buf_len < 1) return fail(DTRAJ_EINVAL, "plan_describe: bad argument");
+    DTRAJ_TRY(cached_plan(u, n_rows, workspace, workspace_bytes, options));
+    PlanText T;
+    T.P = u->plan;
+    T.build();
+    if (T.rc) return T.rc;
+    if ((int64_t)T.s.size() + 1 > buf_len) return fail(DTRAJ_ENOMEM, "plan_describe: %zu bytes needed", T.s.size() + 1);
+    memcpy(buf, T.s.c_str(), T.s.size() + 1);
+    return 0;
+}
+
+extern "C" int dtraj_test_plan_run(dtraj_unet* u, const float* x, int64_t n_rows, int32_t t, const int32_t* row_variant,
+                                   int32_t per_row, void* workspace, int64_t workspace_bytes, int32_t options, int32_t first,
+                                   int32_t last, void* stream) {
+    if (!u || !x || !workspace || (per_row && !row_variant)) return fail(DTRAJ_EINVAL, "plan_run: null argument");
+    DTRAJ_TRY(cached_plan(u, n_rows, workspace, workspace_bytes, options));
+    if (first < 0 || first > last || (size_t)last > u->plan->launches.size())
+        return fail(DTRAJ_EINVAL, "plan_run: launches [%d, %d) outside the plan's %zu", first, last, u->plan->launches.size());
+    const int C = u->d.channels, H = u->d.image_size;
+    return plan_forward(u->plan, x, (int64_t)C * H * H, nullptr, row_variant, per_row ? 0 : t, per_row != 0, (cudaStream_t)stream,
+                        nullptr, (size_t)first, (size_t)last);
 }
 
 extern "C" int dtraj_test_conv(int32_t precision, const float* x0, int32_t c0, const float* x1, int32_t c1, int64_t n, int32_t H,

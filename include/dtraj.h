@@ -326,6 +326,23 @@ int dtraj_test_conv(int32_t precision, const float* x0, int32_t c0, const float*
                     int32_t cout, int32_t ksize, int32_t flags, const float* resid,
                     float* out, void* stream);
 
+/* The forward plan one launch at a time (tests/test_gpu_layers.py).  Both build the plan dtraj_unet_forward would
+ * use for (n_rows, workspace), or reuse the handle's cached one; `options` bit 0 builds it WITHOUT the fused enc1
+ * kernel (k_conv_first, then the generic enc1.conv2 with the CONV_RESX tails), a plan the product never builds for the
+ * supported models.  The cached plan is rebuilt whenever n_rows, the workspace or the options change.
+ * dtraj_test_plan_describe writes NUL-terminated text into buf, one record per line:
+ *   plan R=.. options=.. precision=.. launches=..
+ *   buf name=.. off=.. bytes=.. lo=.. type=f16|f32             every workspace buffer: byte offset, bytes, lo-plane offset
+ *   launch i=.. kind=.. grid=.. flags=.. act=.. tb=.. form=generic|halo1|halo2|posm|none pair=.. split=.. nblk=.. epi=.. name=..
+ *   tensor i=.. role=.. dir=in|out buf=..|x S=.. cp=.. type=..  every map launch i reads or writes (x: the raw frames)
+ * dtraj_test_plan_run enqueues launches [first, last) of that plan on `stream` exactly as the forward does; per_row = 1
+ * is the dtraj_unet_forward_rows form (row_variant then holds t_i * 3 + variant_i and t is ignored). */
+int dtraj_test_plan_describe(dtraj_unet* unet, int64_t n_rows, void* workspace, int64_t workspace_bytes,
+                             int32_t options, char* buf, int64_t buf_len);
+int dtraj_test_plan_run(dtraj_unet* unet, const float* x, int64_t n_rows, int32_t t, const int32_t* row_variant,
+                        int32_t per_row, void* workspace, int64_t workspace_bytes, int32_t options,
+                        int32_t first, int32_t last, void* stream);
+
 /* ------------------------------------------------------------------ diagnostics (tools/, not used by the package's hot path)
  * Kernel-only timing of one conv layer shape on zero-filled buffers allocated inside (tools/conv_bench.py): `iters`
  * launches between one event pair, average milliseconds in *ms_out.  flags: bit0 relu, bit2 residual input, plus the

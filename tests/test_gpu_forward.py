@@ -108,10 +108,11 @@ def test_forward_bench_sized_batch(sf, prec):
 
 
 @pytest.mark.parametrize("C,H", [(1, 16), (3, 32)])
-def test_forward_f16_unfused_first_block(C, H, monkeypatch):
+def test_forward_f16_unfused_first_block(C, H):
     """fp16 mode without the fused enc1 kernel (what first blocks wider than 128 channels take): k_conv_first writing
-    fp16, the generic conv2 with the recomputed 1x1 residual and the pool tail (16x16) or k_pool2_h (32x32)."""
-    monkeypatch.setenv("DTRAJ_NO_ENC1", "1")
+    fp16, the generic conv2 with the recomputed 1x1 residual and the pool tail (16x16) or k_pool2_h (32x32).  The supported
+    models all take the fused kernel, so the plan is built through the test hook with options bit 0."""
+    from test_gpu_layers import CONV_RESX, NO_ENC1, describe
     cfg = Cfg(C, H, 50)
     model = make_model(cfg, 0.3, 13, device="cuda")
     sd = cpu_sd(model)
@@ -119,7 +120,20 @@ def test_forward_f16_unfused_first_block(C, H, monkeypatch):
     x = torch.randn(4, C, H, H)
     variants = torch.tensor([0, 1, 2, 1], dtype=torch.int32)
     eng = UNetEngine.for_model(model, H, 50, "f16")
-    got = eng.forward(x.cuda(), 31, variants.cuda()).cpu().numpy()
+    ws = torch.empty(eng.workspace_bytes(4), dtype=torch.uint8, device="cuda")
+    _, bufs, launches = describe(eng, 4, ws, NO_ENC1)
+    assert launches[0]["kind"] == "FIRST" and [t["type"] for t in launches[0]["tensors"] if t["dir"] == "out"] == ["f16"]
+    assert any(L["kind"] == "CONV_UMMA" and L["flags"] & CONV_RESX for L in launches)
+    assert not any(L["kind"] in ("ENC1", "ENC1H") for L in launches)
+    xd, vd = x.cuda(), variants.cuda()
+    _lib.check(eng.lib.dtraj_test_plan_run(eng.handle, _lib.ptr(xd), 4, 31, _lib.ptr(vd), 0, _lib.ptr(ws), ws.numel(), NO_ENC1,
+                                           0, len(launches), _lib.stream_ptr()))
+    torch.cuda.synchronize()
+    off = bufs["elow"]["off"]
+    elow = ws[off:off + 4 * (H // 2) ** 2 * C * 4].view(torch.float32).view(4, H // 2, H // 2, C)
+    # (eps = bilinear x2 of the half-resolution eps, k_eps_out's job in the product, here in f64)
+    got = torch.nn.functional.interpolate(elow.permute(0, 3, 1, 2).double(), scale_factor=2, mode="bilinear",
+                                          align_corners=True).cpu().numpy()
     tt = torch.full((1,), 31, dtype=torch.long)
     for r in range(4):
         cond = None if variants[r] == 0 else torch.full((1, 1), float(variants[r] - 1))
