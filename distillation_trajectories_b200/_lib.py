@@ -64,6 +64,9 @@ SIGNATURES = {
     "dtraj_wasserstein": (C.c_int, [_P, _P, _I64, _I32, _I32, _P, _P, _I32, _P, _P]),
     "dtraj_metrics_pairs_ragged": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _P, _P, _P, _P]),
     "dtraj_wasserstein_ragged": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _P, _P, _I32, _P, _P]),
+    "dtraj_metrics_pairs_resampled": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _P, _P, _P]),
+    "dtraj_wasserstein_resampled": (C.c_int, [_P, _P, _I64, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _P, _I32, _P,
+                                              _P]),
     "dtraj_unet_forward_rows":(C.c_int, [_P, _P, _I64, _P, _P, _P, _I64, _P]),
     "dtraj_numpy_choice_sets": (C.c_int, [_P, _I32, _I32, _I32, _I32, _P, _P]),
     "dtraj_project": (C.c_int, [_P, _I64, _I32, _P, _P, _I32, _P, _P]),

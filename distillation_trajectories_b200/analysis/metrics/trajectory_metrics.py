@@ -7,9 +7,12 @@ streaming CUDA kernels (``dtraj_metrics_pairs`` / ``dtraj_wasserstein``); the f6
 formulas (log1p / exp / ratios) are evaluated on the host exactly as the reference does, so
 1e-4 parity does not depend on the device's libm.  Teacher and student trajectories of
 different lengths (trajectory_metrics.py:239-279) take ``dtraj_metrics_pairs_ragged`` /
-``dtraj_wasserstein_ragged``, which also compute the path alignment on the device.
+``dtraj_wasserstein_ragged``, which also compute the path alignment on the device.  Student frames of another
+spatial size than the teacher's (trajectory_metrics.py:40-52, resized with bilinear interpolation) take
+``dtraj_metrics_pairs_resampled`` / ``dtraj_wasserstein_resampled``, which read the student at its own size and resize it
+inside the kernels.
 
-Batched API (what the sweep drivers use): ``pair_reductions`` (``pair_reductions_ragged``) +
+Batched API (what the sweep drivers use): ``pair_reductions`` (``pair_reductions_ragged``, ``pair_reductions_resampled``) +
 ``wasserstein_frames`` + ``scalar_metrics_batched`` over [N, L, D] device tensors, or
 ``pair_metrics`` for all three.  ``compute_trajectory_metrics`` keeps the reference's
 list-of-tensors signature and 25-key result; ``compute_trajectory_metrics_many`` returns the
@@ -106,10 +109,39 @@ def pair_reductions_ragged(teacher, student):
     return out
 
 
-def wasserstein_frames(teacher, student, idx=None, idx_set=None):
+def _resampled_shapes(teacher, student, teacher_hw, student_hw, what):
+    """(C, Ht, Wt, Cs, Hs, Ws) of teacher [N, LT, C*Ht*Wt] and student [N, LS, Cs*Hs*Ws]; the library refuses Cs != C."""
+    (Ht, Wt), (Hs, Ws) = (int(v) for v in teacher_hw), (int(v) for v in student_hw)
+    if teacher.dim() != 3 or student.dim() != 3 or teacher.shape[0] != student.shape[0] \
+            or teacher.shape[2] % (Ht * Wt) or student.shape[2] % (Hs * Ws):
+        raise ValueError(f"{what} expects [N, LT, C*Ht*Wt] and [N, LS, C*Hs*Ws] tensors")
+    return teacher.shape[2] // (Ht * Wt), Ht, Wt, student.shape[2] // (Hs * Ws), Hs, Ws
+
+
+def pair_reductions_resampled(teacher, student, teacher_hw, student_hw):
+    """teacher [N, LT, C*Ht*Wt], student [N, LS, C*Hs*Ws] (CUDA fp32, contiguous, max(LT, LS) >= 2) -> device tensor
+    [N, max(LT, LS), 8]: ``pair_reductions_ragged`` of the teacher and the student bilinearly resized to the teacher's
+    (Ht, Wt) with align_corners=True, as F.interpolate does, without a resized copy (dtraj_metrics_pairs_resampled in
+    include/dtraj.h).  For LT == LS columns 0-5 are those of ``pair_reductions``."""
+    lib = _lib.load()
+    teacher, student = _dev(teacher).contiguous(), _dev(student).contiguous()
+    shapes = _resampled_shapes(teacher, student, teacher_hw, student_hw, "pair_reductions_resampled")
+    N, LT, LS = teacher.shape[0], teacher.shape[1], student.shape[1]
+    pos, frac = resample_table(LT, LS)
+    pos, frac = torch.from_numpy(pos).to(teacher.device), torch.from_numpy(frac).to(teacher.device)
+    out = torch.empty(N, max(LT, LS), _lib.METRIC_Q_RAGGED, dtype=torch.float32, device=teacher.device)
+    with torch.cuda.device(teacher.device):
+        _lib.check(lib.dtraj_metrics_pairs_resampled(_lib.ptr(teacher), _lib.ptr(student), N, LT, LS, *shapes, _lib.ptr(pos),
+                                                     _lib.ptr(frac), _lib.ptr(out), _lib.stream_ptr()))
+    return out
+
+
+def wasserstein_frames(teacher, student, idx=None, idx_set=None, frame_hw=None):
     """Per-frame W1 between gathered elements of teacher [N, LT, D] and student [N, LS, D], for the first
     L = min(LT, LS) frames.  ``idx``: int32 [n_sets, L, K] (CUDA) or None for all elements; ``idx_set``: int32 [N]
-    choosing the set per pair.  Returns device [N, L] fp32."""
+    choosing the set per pair.  ``frame_hw`` = ((Ht, Wt), (Hs, Ws)): the student's frames [N, LS, C*Hs*Ws] are of
+    another size and are compared as bilinearly resized to (Ht, Wt) (``idx`` then indexes the teacher's frame, at most
+    1024 elements).  Returns device [N, L] fp32."""
     lib = _lib.load()
     teacher, student = _dev(teacher).contiguous(), _dev(student).contiguous()
     N, LT, D = teacher.shape
@@ -121,7 +153,11 @@ def wasserstein_frames(teacher, student, idx=None, idx_set=None):
     if idx_set is not None:
         idx_set = idx_set.to(teacher.device, torch.int32).contiguous()
     with torch.cuda.device(teacher.device):
-        if LT == LS:
+        if frame_hw is not None:
+            shapes = _resampled_shapes(teacher, student, *frame_hw, "wasserstein_frames")
+            rc = lib.dtraj_wasserstein_resampled(_lib.ptr(teacher), _lib.ptr(student), N, LT, LS, *shapes, _lib.ptr(idx),
+                                                 _lib.ptr(idx_set), K, _lib.ptr(out), _lib.stream_ptr())
+        elif LT == LS:
             rc = lib.dtraj_wasserstein(_lib.ptr(teacher), _lib.ptr(student), N, LT, D, _lib.ptr(idx), _lib.ptr(idx_set),
                                        K, _lib.ptr(out), _lib.stream_ptr())
         else:
@@ -245,24 +281,29 @@ def draw_index_sets(n, numel):
     return np.stack([np.random.choice(numel, K, replace=False) for _ in range(n)]).astype(np.int32)
 
 
-def pair_metrics(teacher, student, idx, pixels, samples=1):
-    """Scalar formulas of ``scalar_metrics_batched`` for G pairs of the same lengths and frame shape.
+def pair_metrics(teacher, student, idx, pixels, samples=1, frame_hw=None):
+    """Scalar formulas of ``scalar_metrics_batched`` for G pairs of the same lengths and frame shapes.
 
-    teacher  device fp32 [G, LT, numel], student [G, LS, numel]: whole frames, a frame's ``samples`` images one
+    teacher  device fp32 [G, LT, numel], student [G, LS, numel_s]: whole frames, a frame's ``samples`` images one
              after another
-    idx      np.int32 [G, min(LT, LS), K] from ``draw_index_sets``, pair by pair
+    idx      np.int32 [G, min(LT, LS), K] from ``draw_index_sets``, pair by pair (teacher-frame indices)
+    frame_hw ((Ht, Wt), (Hs, Ws)) when the student's images are of another size: they are compared as bilinearly
+             resized to the teacher's (trajectory_metrics.py:40-52), numel_s = numel * Hs * Ws / (Ht * Wt)
     The reductions run per image and are added in f64 (torch.norm over a whole [B, C, H, W] frame).
     """
     G, LT, numel = teacher.shape
     LS = student.shape[1]
-    per_image = lambda x: x.reshape(G, x.shape[1], samples, numel // samples).transpose(1, 2) \
-        .reshape(G * samples, x.shape[1], numel // samples)
-    reduce = pair_reductions if LT == LS else pair_reductions_ragged
+    per_image = lambda x: x.reshape(G, x.shape[1], samples, x.shape[2] // samples).transpose(1, 2) \
+        .reshape(G * samples, x.shape[1], x.shape[2] // samples)
+    if frame_hw is not None:
+        reduce = lambda t, s: pair_reductions_resampled(t, s, *frame_hw)
+    else:
+        reduce = pair_reductions if LT == LS else pair_reductions_ragged
     red = reduce(per_image(teacher), per_image(student)).cpu().numpy()
     red = red.reshape(G, samples, *red.shape[1:]).astype(np.float64).sum(axis=1).astype(np.float32)
     all_elements = idx.shape[-1] == numel
     w1 = wasserstein_frames(teacher, student, None if all_elements else torch.from_numpy(idx),
-                            None if all_elements else torch.arange(G, dtype=torch.int32)).cpu().numpy()
+                            None if all_elements else torch.arange(G, dtype=torch.int32), frame_hw).cpu().numpy()
     return scalar_metrics_batched(red, w1, pixels, numel, (LT, LS))
 
 
@@ -296,34 +337,27 @@ def _metrics_dict(sm, j):
 def compute_trajectory_metrics(teacher_trajectory, student_trajectory, config=None):
     """Metrics between one teacher and one student trajectory (lists of [B, C, H, W] tensors or
     (tensor, t) tuples).  Same 25 keys, value types and numpy-global-RNG use as the reference."""
-    T = _images(teacher_trajectory)
-    S = _images(student_trajectory)
-    if T[-1].shape != S[-1].shape and T[-1].shape[2:] != S[-1].shape[2:]:
-        # trajectory_metrics.py:40-52: bilinear (align_corners) resize of every student frame
-        dev = _pick_device(T + S)
-        S = [torch.nn.functional.interpolate(s.to(dev), size=T[0].shape[2:], mode="bilinear", align_corners=True)
-             for s in S]
-    return compute_trajectory_metrics_many([(T, S)])[0]
+    return compute_trajectory_metrics_many([(teacher_trajectory, student_trajectory)])[0]
 
 
 def compute_trajectory_metrics_many(pairs):
     """``compute_trajectory_metrics`` of every (teacher, student) pair of ``pairs``, in order.  Pairs with the same
-    lengths and frame shape share one launch of each kernel; the results, and the global numpy RNG's state afterwards,
-    are those of calling ``compute_trajectory_metrics`` on each pair in turn."""
+    lengths and frame shapes share one launch of each kernel; the results, and the global numpy RNG's state afterwards,
+    are those of calling ``compute_trajectory_metrics`` on each pair in turn.  A student whose frames differ from the
+    teacher's in H x W is compared as resized to the teacher's (trajectory_metrics.py:40-52), inside the kernels."""
     out = [None] * len(pairs)
     groups = {}
     for k, (t, s) in enumerate(pairs):
         T, S = _images(t), _images(s)
-        if T[-1].shape != S[-1].shape and T[-1].shape[2:] != S[-1].shape[2:]:
-            out[k] = compute_trajectory_metrics(T, S)          # student frames resized on their own
-            continue
         idx = draw_index_sets(min(len(T), len(S)), T[0].numel())
-        groups.setdefault((len(T), len(S), tuple(T[0].shape)), []).append((k, T, S, idx))
-    for (_, _, shape), items in groups.items():
+        groups.setdefault((len(T), len(S), tuple(T[0].shape), tuple(S[0].shape)), []).append((k, T, S, idx))
+    for (_, _, shape, s_shape), items in groups.items():
         dev = _pick_device(items[0][1] + items[0][2])
         ft = torch.stack([_stack_frames(T, dev) for _, T, _, _ in items])
         fs = torch.stack([_stack_frames(S, dev) for _, _, S, _ in items])
-        sm = pair_metrics(ft, fs, np.stack([it[3] for it in items]), shape[2] * shape[3], samples=shape[0])
+        resized = shape != s_shape and shape[2:] != s_shape[2:]
+        sm = pair_metrics(ft, fs, np.stack([it[3] for it in items]), shape[2] * shape[3], samples=shape[0],
+                          frame_hw=(shape[2:], s_shape[2:]) if resized else None)
         for j, it in enumerate(items):
             out[it[0]] = _metrics_dict(sm, j)
     return out

@@ -1027,6 +1027,22 @@ extern "C" int dtraj_wasserstein_ragged(const float* teacher, const float* stude
     return launch_wasserstein(teacher, student, N, LT, LS, D, idx, idx_set, K, out, (cudaStream_t)stream);
 }
 
+extern "C" int dtraj_metrics_pairs_resampled(const float* teacher, const float* student, int64_t N, int32_t LT, int32_t LS,
+                                             int32_t C, int32_t Ht, int32_t Wt, int32_t Cs, int32_t Hs, int32_t Ws,
+                                             const int32_t* rs_pos, const float* rs_frac, float* out, void* stream) {
+    if (N == 0) return 0;
+    if (!teacher || !student || !rs_pos || !rs_frac || !out || N < 0) return fail(DTRAJ_EINVAL, "metrics_resampled: bad argument");
+    return launch_metrics_pairs_resampled(teacher, student, N, LT, LS, C, Ht, Wt, Cs, Hs, Ws, rs_pos, rs_frac, out, (cudaStream_t)stream);
+}
+
+extern "C" int dtraj_wasserstein_resampled(const float* teacher, const float* student, int64_t N, int32_t LT, int32_t LS,
+                                           int32_t C, int32_t Ht, int32_t Wt, int32_t Cs, int32_t Hs, int32_t Ws,
+                                           const int32_t* idx, const int32_t* idx_set, int32_t K, float* out, void* stream) {
+    if (N == 0) return 0;
+    if (!teacher || !student || !out || N < 0) return fail(DTRAJ_EINVAL, "wasserstein_resampled: bad argument");
+    return launch_wasserstein_resampled(teacher, student, N, LT, LS, C, Ht, Wt, Cs, Hs, Ws, idx, idx_set, K, out, (cudaStream_t)stream);
+}
+
 extern "C" int dtraj_numpy_choice_sets(const uint32_t* seeds, int32_t n_seeds, int32_t L, int32_t D, int32_t K, int32_t* out, void* stream) {
     if (n_seeds == 0) return 0;
     if (!seeds || !out) return fail(DTRAJ_EINVAL, "numpy_choice_sets: null argument");

@@ -5,6 +5,7 @@
 //   Wasserstein per frame:          analysis/metrics/trajectory_metrics.py:296-312
 #pragma once
 #include <cstdlib>
+#include <type_traits>
 #include "common.cuh"
 
 namespace dtraj {
@@ -145,11 +146,17 @@ inline int launch_metrics_pairs(const float* T, const float* S, int64_t N, int L
 // (p non-decreasing, 0 <= p_j <= L_long - 2), and at the last long frame at the latest.
 constexpr int kRaggedQ = 8;
 
-template <int K>
+// Frame source of k_metrics_pairs_ragged.  DirectFrames reads [N, LT, D] and [N, LS, D] in place through the pointers
+// the kernel forms itself; ResampledFrames (below) reads a student of another frame size through the bilinear resize.
+struct DirectFrames {
+    static constexpr bool kInPlace = true;
+};
+
+template <int K, class Frames>
 __global__ void __launch_bounds__(256) k_metrics_pairs_ragged(const float* __restrict__ teacher, const float* __restrict__ student,
                                                               int64_t N, int LT, int LS, int D4, int G,
                                                               const int32_t* __restrict__ rs_pos, const float* __restrict__ rs_frac,
-                                                              float* __restrict__ out) {
+                                                              float* __restrict__ out, Frames frames) {
     extern __shared__ float part[];          // [pairs_per_block][Lmax][warps_per_group][5]
     const int ppb = 256 / G, wpg = G / 32 > 0 ? G / 32 : 1;
     const int g = threadIdx.x / G, tg = threadIdx.x % G;
@@ -164,11 +171,15 @@ __global__ void __launch_bounds__(256) k_metrics_pairs_ragged(const float* __res
     const float4* Tb = reinterpret_cast<const float4*>(teacher) + (active ? n : 0) * (int64_t)LT * D4;
     const float4* Sb = reinterpret_cast<const float4*>(student) + (active ? n : 0) * (int64_t)LS * D4;
     const float4* Shb = t_long ? Sb : Tb;
-    auto load = [&](const float4* base, int i, bool ok, float4* v) {
+    // stu: base is the student's trajectory
+    auto load = [&](const float4* base, bool stu, int i, bool ok, float4* v) {
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             const int e = tg + k * G;
-            v[k] = (ok && active && e < D4) ? ld_stream4(reinterpret_cast<const float*>(base + (int64_t)i * D4 + e)) : zero4;
+            if constexpr (Frames::kInPlace)
+                v[k] = (ok && active && e < D4) ? ld_stream4(reinterpret_cast<const float*>(base + (int64_t)i * D4 + e)) : zero4;
+            else
+                v[k] = (ok && active && e < D4) ? frames.load(teacher, student, stu, n, LT, LS, i, e, D4) : zero4;
         }
     };
     auto sq4 = [](float4 a) { return a.x * a.x + a.y * a.y + a.z * a.z + a.w * a.w; };
@@ -179,16 +190,16 @@ __global__ void __launch_bounds__(256) k_metrics_pairs_ragged(const float* __res
         return make_float4(e * a.x + f * b.x, e * a.y + f * b.y, e * a.z + f * b.z, e * a.w + f * b.w);
     };
 
-    load(Tb, 0, true, nxtT);
-    load(Sb, 0, true, nxtS);
+    load(Tb, false, 0, true, nxtT);
+    load(Sb, true, 0, true, nxtS);
     float endT = 0.f, endS = 0.f, endTS = 0.f;
     int j = 0;                               // next short frame of the path-alignment term
     for (int i = 0; i < Lmax; ++i) {
         float4 curT[K], curS[K];
 #pragma unroll
         for (int k = 0; k < K; ++k) { curT[k] = nxtT[k]; curS[k] = nxtS[k]; }
-        load(Tb, i + 1, i + 1 < LT, nxtT);
-        load(Sb, i + 1, i + 1 < LS, nxtS);
+        load(Tb, false, i + 1, i + 1 < LT, nxtT);
+        load(Sb, true, i + 1, i + 1 < LS, nxtS);
         const bool inT = i < LT, inS = i < LS;
         float d2 = 0.f, vt2 = 0.f, vs2 = 0.f, dot = 0.f;
 #pragma unroll
@@ -200,24 +211,24 @@ __global__ void __launch_bounds__(256) k_metrics_pairs_ragged(const float* __res
             }
         }
         if (i == LT - 1) {                   // frame 0 is re-read rather than held in registers for the whole walk
-            load(Tb, 0, true, sh);
+            load(Tb, false, 0, true, sh);
 #pragma unroll
             for (int k = 0; k < K; ++k) endT += sq4(sub4(curT[k], sh[k]));
         }
         if (i == LS - 1) {
-            load(Sb, 0, true, sh);
+            load(Sb, true, 0, true, sh);
 #pragma unroll
             for (int k = 0; k < K; ++k) endS += sq4(sub4(curS[k], sh[k]));
         }
         if (i == Lmax - 1) {                 // the long trajectory's last frame against the short one's (re-read)
-            load(Shb, Ln - 1, true, sh);
+            load(Shb, t_long, Ln - 1, true, sh);
 #pragma unroll
             for (int k = 0; k < K; ++k) endTS += sq4(sub4(t_long ? curT[k] : curS[k], sh[k]));
         }
         // path alignment: every short frame j whose interval [p_j, p_j + 1] ends at this long frame
         while (i > 0 && j < Ln && (__ldg(rs_pos + j) <= i - 1 || i == Lmax - 1)) {
             const float f = __ldg(rs_frac + j);
-            load(Shb, j, true, sh);
+            load(Shb, t_long, j, true, sh);
             float r2 = 0.f;
 #pragma unroll
             for (int k = 0; k < K; ++k)
@@ -260,25 +271,23 @@ __global__ void __launch_bounds__(256) k_metrics_pairs_ragged(const float* __res
     }
 }
 
-inline int launch_metrics_pairs_ragged(const float* T, const float* S, int64_t N, int LT, int LS, int D,
-                                       const int32_t* rs_pos, const float* rs_frac, float* out, cudaStream_t st) {
-    if (D % 4 != 0 || D <= 0 || LT < 1 || LS < 1 || (LT < 2 && LS < 2))
-        return fail(DTRAJ_EINVAL, "metrics_ragged: D=%d must be a positive multiple of 4, LT=%d, LS=%d >= 1 and one of them >= 2", D, LT, LS);
-    const int D4 = D / 4;
+// max(LT, LS) >= 2 and D4 <= 1024 float4 per group are checked by the callers.
+template <class Frames>
+inline int launch_ragged_walk(const float* T, const float* S, int64_t groups, int LT, int LS, int D4, const int32_t* rs_pos,
+                              const float* rs_frac, float* out, Frames frames, const char* who, cudaStream_t st) {
     int G = 32;
     while (G < 256 && (D4 + G - 1) / G > 3) G *= 2;
     const int K = (D4 + G - 1) / G;
-    if (K > 4) return fail(DTRAJ_EINVAL, "metrics_ragged: D=%d too large (max 4096)", D);
     const int ppb = 256 / G, wpg = G / 32, Lmax = LT > LS ? LT : LS;
     const size_t smem = (size_t)ppb * Lmax * wpg * 5 * sizeof(float);
-    if (smem > 200 * 1024) return fail(DTRAJ_EINVAL, "metrics_ragged: max(LT, LS)=%d too large", Lmax);
-    if (N == 0) return 0;
-    const unsigned grid = (unsigned)((N + ppb - 1) / ppb);
+    if (smem > 200 * 1024) return fail(DTRAJ_EINVAL, "%s: max(LT, LS)=%d too large", who, Lmax);
+    if (groups == 0) return 0;
+    const unsigned grid = (unsigned)((groups + ppb - 1) / ppb);
 #define DTRAJ_MPR(KK)                                                                             \
     {                                                                                             \
         if (smem > 48 * 1024)                                                                     \
-            DTRAJ_CUDA(cudaFuncSetAttribute(k_metrics_pairs_ragged<KK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        k_metrics_pairs_ragged<KK><<<grid, 256, smem, st>>>(T, S, N, LT, LS, D4, G, rs_pos, rs_frac, out); \
+            DTRAJ_CUDA(cudaFuncSetAttribute(k_metrics_pairs_ragged<KK, Frames>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        k_metrics_pairs_ragged<KK, Frames><<<grid, 256, smem, st>>>(T, S, groups, LT, LS, D4, G, rs_pos, rs_frac, out, frames); \
     }
     switch (K) {
         case 1: DTRAJ_MPR(1); break;
@@ -289,6 +298,112 @@ inline int launch_metrics_pairs_ragged(const float* T, const float* S, int64_t N
 #undef DTRAJ_MPR
     DTRAJ_LAUNCH_CHECK();
     return 0;
+}
+
+inline int launch_metrics_pairs_ragged(const float* T, const float* S, int64_t N, int LT, int LS, int D,
+                                       const int32_t* rs_pos, const float* rs_frac, float* out, cudaStream_t st) {
+    if (D % 4 != 0 || D <= 0 || LT < 1 || LS < 1 || (LT < 2 && LS < 2))
+        return fail(DTRAJ_EINVAL, "metrics_ragged: D=%d must be a positive multiple of 4, LT=%d, LS=%d >= 1 and one of them >= 2", D, LT, LS);
+    if (D > 4096) return fail(DTRAJ_EINVAL, "metrics_ragged: D=%d too large (max 4096)", D);
+    return launch_ragged_walk(T, S, N, LT, LS, D / 4, rs_pos, rs_frac, out, DirectFrames{}, "metrics_ragged", st);
+}
+
+// ---------------------------------------------------------------- student frames of another size
+// compute_trajectory_metrics resizes every student frame to the teacher's H x W when the two differ
+// (analysis/metrics/trajectory_metrics.py:40-52: F.interpolate(mode="bilinear", align_corners=True)).  The kernels below
+// read the student at its own size and form the resized value of each teacher element on the fly, with torch's
+// upsample_bilinear2d arithmetic in fp32: scale = (Hs - 1) / (Ht - 1) (0 when Ht == 1), src = scale * y, y0 = (int)src,
+// y1 = y0 + (y0 < Hs - 1), ly = src - y0, the same along x, and four taps.  The resize has no antialiasing, so
+// downsampling is the same four-tap formula.  No resized copy is ever written.
+struct Bilinear {
+    int Ht, Wt, Hs, Ws;
+    float sh, sw;
+    __host__ Bilinear(int ht, int wt, int hs, int ws)
+        : Ht(ht), Wt(wt), Hs(hs), Ws(ws), sh(ht > 1 ? (float)(hs - 1) / (float)(ht - 1) : 0.f),
+          sw(wt > 1 ? (float)(ws - 1) / (float)(wt - 1) : 0.f) {}
+    // the resized value at teacher element (c, y, x) of the student frame s [C, Hs, Ws]
+    __device__ __forceinline__ float at(const float* s, int c, int y, int x) const {
+        const float fy = sh * (float)y, fx = sw * (float)x;
+        const int y0 = (int)fy, x0 = (int)fx;
+        const int y1 = y0 + (y0 < Hs - 1), x1 = x0 + (x0 < Ws - 1);
+        const float ly = fy - (float)y0, lx = fx - (float)x0;
+        const float* r0 = s + ((int64_t)c * Hs + y0) * Ws;
+        const float* r1 = s + ((int64_t)c * Hs + y1) * Ws;
+        return (1.f - ly) * ((1.f - lx) * __ldg(r0 + x0) + lx * __ldg(r0 + x1)) +
+               ly * ((1.f - lx) * __ldg(r1 + x0) + lx * __ldg(r1 + x1));
+    }
+};
+
+// Frame source of k_metrics_pairs_ragged for teacher [N, LT, C, Ht, Wt] and student [N, LS, C, Hs, Ws].  A teacher frame
+// wider than one group's 4096 elements is cut into `parts` bands of whole teacher rows: group n covers band n % parts of
+// pair n / parts and reads, through the resize, exactly the student rows its band needs.  Wt % 4 == 0, so the four
+// elements of a teacher float4 lie on one row.  Teacher loads stream past L1 (ld.global.nc.L1::no_allocate); the
+// student's taps, which neighbouring elements share, go through the read-only cache.
+struct ResampledFrames {
+    static constexpr bool kInPlace = false;
+    Bilinear bl;
+    int parts, HWt;
+    int64_t Dt, Ds;                          // teacher and student frame sizes in floats
+    // float4 e (of the band's D4) of frame i of group n's teacher or student
+    __device__ __forceinline__ float4 load(const float* teacher, const float* student, bool stu, int64_t n, int LT, int LS, int i,
+                                           int e, int D4) const {
+        const int64_t pr = n / parts;
+        const int d = (int)(n - pr * parts) * 4 * D4 + 4 * e;   // teacher element of the float4's first lane
+        if (!stu) return ld_stream4(teacher + (pr * LT + i) * Dt + d);
+        const float* f = student + (pr * LS + i) * Ds;
+        const int c = d / HWt, r = d - c * HWt, y = r / bl.Wt, x = r - y * bl.Wt;
+        return make_float4(bl.at(f, c, y, x), bl.at(f, c, y, x + 1), bl.at(f, c, y, x + 2), bl.at(f, c, y, x + 3));
+    }
+};
+
+// out[n][m] = sum over the parts of part[n][p][m], added in f64 in part order
+__global__ void __launch_bounds__(256) k_sum_parts(const float* __restrict__ part, int64_t N, int parts, int M, float* __restrict__ out) {
+    for (int64_t o = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; o < N * M; o += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t n = o / M, m = o - n * M;
+        double s = 0.0;
+        for (int p = 0; p < parts; ++p) s += (double)part[(n * parts + p) * M + m];
+        out[o] = (float)s;
+    }
+}
+
+constexpr int kResampledMaxElems = 16384;    // C * Ht * Wt of a teacher frame for the reductions (4 x 64 x 64)
+
+// teacher [.., C, Ht, Wt] against student [.., Cs, Hs, Ws]; frames of at most max_elems teacher elements
+inline int check_resampled(const char* who, int LT, int LS, int C, int Ht, int Wt, int Cs, int Hs, int Ws, int64_t max_elems) {
+    if (LT < 1 || LS < 1 || C < 1 || Ht < 1 || Wt < 1 || Cs < 1 || Hs < 1 || Ws < 1)
+        return fail(DTRAJ_EINVAL, "%s: LT=%d, LS=%d and the sizes C=%d, Ht=%d, Wt=%d, Cs=%d, Hs=%d, Ws=%d must be positive", who, LT, LS,
+                    C, Ht, Wt, Cs, Hs, Ws);
+    if (Cs != C) return fail(DTRAJ_EINVAL, "%s: teacher has %d channels, student %d", who, C, Cs);
+    if ((int64_t)C * Ht * Wt > max_elems)
+        return fail(DTRAJ_EINVAL, "%s: teacher frame C*Ht*Wt=%lld too large (max %lld)", who, (long long)C * Ht * Wt, (long long)max_elems);
+    if ((int64_t)C * Hs * Ws > 0x7fffffffLL) return fail(DTRAJ_EINVAL, "%s: student frame C*Hs*Ws too large", who);
+    return 0;
+}
+
+inline int launch_metrics_pairs_resampled(const float* T, const float* S, int64_t N, int LT, int LS, int C, int Ht, int Wt, int Cs,
+                                          int Hs, int Ws, const int32_t* rs_pos, const float* rs_frac, float* out, cudaStream_t st) {
+    DTRAJ_TRY(check_resampled("metrics_resampled", LT, LS, C, Ht, Wt, Cs, Hs, Ws, kResampledMaxElems));
+    if (LT < 2 && LS < 2) return fail(DTRAJ_EINVAL, "metrics_resampled: one of LT=%d, LS=%d must be >= 2", LT, LS);
+    if (Wt % 4 != 0) return fail(DTRAJ_EINVAL, "metrics_resampled: Wt=%d must be a multiple of 4", Wt);
+    const int rows = C * Ht;
+    int parts = 1;                           // the fewest bands of whole rows of at most 4096 elements
+    while (parts <= rows && (rows % parts || (rows / parts) * Wt > 4096)) ++parts;
+    if (parts > rows) return fail(DTRAJ_EINVAL, "metrics_resampled: a teacher row of Wt=%d is wider than 4096", Wt);
+    ResampledFrames fr{Bilinear(Ht, Wt, Hs, Ws), parts, Ht * Wt, (int64_t)C * Ht * Wt, (int64_t)C * Hs * Ws};
+    const int D4 = rows / parts * Wt / 4, Lmax = LT > LS ? LT : LS;
+    if (N == 0) return 0;
+    if (parts == 1) return launch_ragged_walk(T, S, N, LT, LS, D4, rs_pos, rs_frac, out, fr, "metrics_resampled", st);
+    float* part = nullptr;
+    DTRAJ_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&part), (size_t)N * parts * Lmax * kRaggedQ * sizeof(float), st));
+    int rc = launch_ragged_walk(T, S, N * parts, LT, LS, D4, rs_pos, rs_frac, part, fr, "metrics_resampled", st);
+    if (rc == 0) {
+        const int64_t want = (N * Lmax * kRaggedQ + 255) / 256;
+        k_sum_parts<<<(unsigned)(want < 8 * kNumSMs ? want : 8 * kNumSMs), 256, 0, st>>>(part, N, parts, Lmax * kRaggedQ, out);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) rc = fail(DTRAJ_ECUDA, "metrics_resampled: launch -> %s", cudaGetErrorString(e));
+    }
+    DTRAJ_CUDA(cudaFreeAsync(part, st));
+    return rc;
 }
 
 // 1-d Wasserstein distance between K gathered elements of T_i and S_i: for equal-size
@@ -375,24 +490,43 @@ __device__ __forceinline__ void warp_bitonic_sort(float (&v)[E], int lane) {
     }
 }
 
-template <int E>
+// Student element source of k_wasserstein_warp: DirectSample reads element el of a student frame of the teacher's size,
+// ResampledSample the resized value at teacher element el of a student [C, Hs, Ws] (the index sets are teacher-frame
+// indices, as the reference draws them after resizing).
+struct DirectSample {
+    __device__ __forceinline__ const float* frame(const float* student, int64_t f, int D) const { return student + f * D; }
+    __device__ __forceinline__ float at(const float* s, int el) const { return __ldg(s + el); }
+};
+
+struct ResampledSample {
+    Bilinear bl;
+    int64_t Ds;                              // student frame size in floats
+    __device__ __forceinline__ const float* frame(const float* student, int64_t f, int /*D*/) const { return student + f * Ds; }
+    __device__ __forceinline__ float at(const float* s, int el) const {
+        const int hw = bl.Ht * bl.Wt, c = el / hw, r = el - c * hw, y = r / bl.Wt;
+        return bl.at(s, c, y, r - y * bl.Wt);
+    }
+};
+
+template <int E, class Student>
 __global__ void __launch_bounds__(256) k_wasserstein_warp(const float* __restrict__ teacher, const float* __restrict__ student,
                                                           int64_t NL, int L, int LT, int LS, int D, const int32_t* __restrict__ idx,
-                                                          const int32_t* __restrict__ idx_set, int K, float* __restrict__ out) {
+                                                          const int32_t* __restrict__ idx_set, int K, float* __restrict__ out,
+                                                          Student stu) {
     const int lane = threadIdx.x & 31;
     const int64_t pf = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);    // n*L + i
     if (pf >= NL) return;
     const int64_t n = pf / L;
     const int i = (int)(pf - n * L);
     const float* t = teacher + (n * LT + i) * D;
-    const float* s = student + (n * LS + i) * D;
+    const float* s = stu.frame(student, n * LS + i, D);
     const int32_t* ix = idx ? idx + ((int64_t)(idx_set ? idx_set[n] : 0) * L + i) * K : nullptr;
     float a[E], b[E];
 #pragma unroll
     for (int e = 0; e < E; ++e) {
         const int k = lane * E + e;
         a[e] = INFINITY; b[e] = INFINITY;
-        if (k < K) { const int el = ix ? __ldg(ix + k) : k; a[e] = __ldg(t + el); b[e] = __ldg(s + el); }
+        if (k < K) { const int el = ix ? __ldg(ix + k) : k; a[e] = __ldg(t + el); b[e] = stu.at(s, el); }
     }
     warp_bitonic_sort<E>(a, lane);
     warp_bitonic_sort<E>(b, lane);
@@ -462,9 +596,11 @@ inline int launch_project(const float* x, int64_t F, int D, const float* comps, 
 }
 
 // Frames i < L = min(LT, LS) of pairs whose teacher holds LT frames and student LS frames ([N, LT, D] / [N, LS, D], read in
-// place); idx is [n_sets, L, K] and out [N, L].  LT == LS is the equal-length form.
+// place, or a student of another frame size through ResampledSample); idx is [n_sets, L, K] and out [N, L].  LT == LS is
+// the equal-length form.  The block-per-frame form for K > 1024 reads students of the teacher's size only.
+template <class Student = DirectSample>
 inline int launch_wasserstein(const float* T, const float* S, int64_t N, int LT, int LS, int D, const int32_t* idx,
-                              const int32_t* idx_set, int K, float* out, cudaStream_t st) {
+                              const int32_t* idx_set, int K, float* out, cudaStream_t st, Student stu = {}) {
     const int L = LT < LS ? LT : LS;
     if (L < 1) return fail(DTRAJ_EINVAL, "wasserstein: LT=%d and LS=%d must be >= 1", LT, LS);
     if (K < 1 || K > D || K > 4096) return fail(DTRAJ_EINVAL, "wasserstein: K=%d out of range (D=%d)", K, D);
@@ -476,18 +612,29 @@ inline int launch_wasserstein(const float* T, const float* S, int64_t N, int LT,
     const int64_t NL = N * L;
     const unsigned wgrid = (unsigned)((NL + 7) / 8);
     if (P <= 256) {
-        k_wasserstein_warp<8><<<wgrid, 256, 0, st>>>(T, S, NL, L, LT, LS, D, idx, idx_set, K, out);
+        k_wasserstein_warp<8, Student><<<wgrid, 256, 0, st>>>(T, S, NL, L, LT, LS, D, idx, idx_set, K, out, stu);
         DTRAJ_LAUNCH_CHECK();
         return 0;
     }
     if (P <= 1024) {
-        k_wasserstein_warp<32><<<wgrid, 256, 0, st>>>(T, S, NL, L, LT, LS, D, idx, idx_set, K, out);
+        k_wasserstein_warp<32, Student><<<wgrid, 256, 0, st>>>(T, S, NL, L, LT, LS, D, idx, idx_set, K, out, stu);
         DTRAJ_LAUNCH_CHECK();
         return 0;
     }
+    if (!std::is_same<Student, DirectSample>::value) return fail(DTRAJ_EINVAL, "wasserstein: K=%d > 1024 with a resampled student", K);
     k_wasserstein<<<(unsigned)(N * L), 256, 2 * P * sizeof(float), st>>>(T, S, L, LT, LS, D, idx, idx_set, K, P, out);
     DTRAJ_LAUNCH_CHECK();
     return 0;
+}
+
+// Frames of any size with int32 element indices: W1 gathers at most 1024 elements of a frame, so, unlike the reductions,
+// it holds no frame in registers (C may count the images of a [B, C, H, W] frame times their channels).
+inline int launch_wasserstein_resampled(const float* T, const float* S, int64_t N, int LT, int LS, int C, int Ht, int Wt, int Cs,
+                                        int Hs, int Ws, const int32_t* idx, const int32_t* idx_set, int K, float* out, cudaStream_t st) {
+    DTRAJ_TRY(check_resampled("wasserstein_resampled", LT, LS, C, Ht, Wt, Cs, Hs, Ws, 0x7fffffffLL));
+    if (K > 1024) return fail(DTRAJ_EINVAL, "wasserstein_resampled: K=%d out of range (max 1024)", K);
+    return launch_wasserstein(T, S, N, LT, LS, C * Ht * Wt, idx, idx_set, K, out, st,
+                              ResampledSample{Bilinear(Ht, Wt, Hs, Ws), (int64_t)C * Hs * Ws});
 }
 
 // ---------------------------------------------------------------- Wasserstein subsample indices on the device

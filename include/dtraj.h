@@ -273,6 +273,46 @@ int dtraj_wasserstein_ragged(const float* teacher, const float* student,
                              float* out, void* stream);
 
 /*
+ * Student frames of another spatial size than the teacher's, N pairs in one launch: the branch of
+ * compute_trajectory_metrics that bilinearly resizes every student frame to the teacher's H x W
+ * (trajectory_metrics.py:40-52, F.interpolate(align_corners=True); a student sampled at another
+ * resolution).  The student is read at its own size and resized on the fly with torch's
+ * upsample_bilinear2d arithmetic in fp32 (four taps, upsampling or downsampling); no resized copy
+ * is written.
+ *   teacher  dev [N, LT, C, Ht, Wt] fp32,  student  dev [N, LS, Cs, Hs, Ws] fp32
+ *            (Cs == C, C*Ht*Wt <= 16384, Wt a multiple of 4, max(LT, LS) >= 2)
+ *   rs_pos, rs_frac  the path-alignment table of dtraj_metrics_pairs_ragged
+ *   out      dev [N, max(LT, LS), 8] fp32: the layout of dtraj_metrics_pairs_ragged, every student
+ *            frame taken as resized (velocities, start-to-end distance, endpoint and alignment
+ *            terms included); for LT == LS columns 0-5 are those of dtraj_metrics_pairs.
+ * Teacher frames of more than 4096 elements are cut into bands of whole teacher rows, reduced
+ * separately (each band reads the student rows it needs) and added in f64.
+ * Algorithmic bytes 4 * N * (C*Ht*Wt * LT + C*Hs*Ws * LS).  Requested: the teacher frame reads of
+ * the ragged walk at 4 bytes per teacher element, and the student's at 16 (four taps per teacher
+ * element, through the read-only cache that neighbouring elements share).
+ * DTRAJ_EINVAL for Cs != C, a non-positive size or C*Ht*Wt > 16384.
+ */
+int dtraj_metrics_pairs_resampled(const float* teacher, const float* student,
+                                  int64_t N, int32_t LT, int32_t LS,
+                                  int32_t C, int32_t Ht, int32_t Wt, int32_t Cs, int32_t Hs, int32_t Ws,
+                                  const int32_t* rs_pos, const float* rs_frac, float* out, void* stream);
+
+/*
+ * dtraj_wasserstein(_ragged) for a student of another frame size: the distances of the first
+ * n = min(LT, LS) frames, the student value of teacher element e being the resized one.
+ *   idx  dev int32 [n_idx_sets, n, K] teacher-frame indices (the reference draws them after
+ *        resizing), or NULL for K == C*Ht*Wt;  K <= 1024;  out dev [N, n] fp32.
+ * C may count the images of a [B, C, H, W] frame times their channels.  The frame holds no
+ * register tile here, so the 16384 limit of the reductions does not apply.
+ * DTRAJ_EINVAL for Cs != C or a non-positive size.
+ */
+int dtraj_wasserstein_resampled(const float* teacher, const float* student,
+                                int64_t N, int32_t LT, int32_t LS,
+                                int32_t C, int32_t Ht, int32_t Wt, int32_t Cs, int32_t Hs, int32_t Ws,
+                                const int32_t* idx, const int32_t* idx_set, int32_t K,
+                                float* out, void* stream);
+
+/*
  * The subsample index sets compute_trajectory_metrics draws for frames larger than 1000 elements
  * (trajectory_metrics.py:301-306: np.random.choice(D, K, replace=False) per frame, from the global numpy RNG that
  * compare_trajectories' callers left at seed + 1, analysis/trajectory_engine.py:91-93), generated on the device: numpy's
